@@ -22,6 +22,15 @@ reset + tile-FIM kernel) + gradient-descent path extraction from a fixed start.
            with its own goal -- independent queries, no data-path collective ("weak").
 
 --impl reference times the UNMODIFIED reference (oracle/_ref) on the host cores.
+
+--dump-outputs DIR writes, after the timed steps, what the last step of the headline arm handed
+its caller: DIR/total_cost.npy (the total-cost matrix, -1 where unreached as getTotalCostMatrix
+delivers it; float64, rows and columns taken with a fixed stride so that it stays under 48 MB:
+every 2nd at 4096^2) and DIR/path.npy (the waypoints, float64).  The inputs depend on --size and --seed only, so two
+builds run with the same arguments can be compared array for array.  Compare with a tolerance:
+the solver's update order varies between runs, and so do the last bits (two runs of one build
+on a B200 differed by at most 3.6e-15 relative on the total cost and 1e-11 on the waypoints,
+with the same unreached cells).
 """
 import argparse
 import json
@@ -36,6 +45,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: leave no __pycache__ in it
 
 METRIC = "plans_per_s"
 UNIT = "plans/s"
@@ -62,7 +72,14 @@ def parse_args():
     ap.add_argument("--queries", type=int, default=1024)
     ap.add_argument("--batch", type=int, default=64)
     ap.add_argument("--seed", type=int, default=20261018)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed plan4096 step as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and (a.impl != "b200" or (a.workload != "all" and "plan4096" not in a.workload.split(","))):
+        ap.error("--dump-outputs needs the b200 plan4096 workload")
+    return a
 
 
 def dist_env():
@@ -169,7 +186,6 @@ def run_reference(args):
         make = lambda: lib.DyMuPathPlanner(1.0, 1.5, 2.0, 1)
         kind = "reference"
     else:
-        oracle.build(ref=False, port=True)
         make = lambda: oracle.Port(1.0, 1.5, 2.0, 1)
         kind = "port"
     planners, goals = [], []
@@ -260,7 +276,6 @@ def cpu_baseline_leg(pkg, elev, terr, lut, slopes, locs, n):
         p = oracle.reference().DyMuPathPlanner(1.0, 1.5, 2.0, 1)
         kind = "reference"
     else:
-        oracle.build(ref=False, port=True)
         p = oracle.Port(1.0, 1.5, 2.0, 1)
         kind = "port"
     p.initGlobalLayer(1.0, 0.1, crop, crop)
@@ -444,11 +459,11 @@ def headline_plan4096(args, D, pkg, affinity):
         st = dev.solve_total_cost([goal])
         wps, status = dev.extract_global_path(float(start[0]), float(start[1]), 0.4, goal[0],
                                               goal[1])
-        return st, len(wps), status
+        return st, wps, status
 
     # ---- resident-input arm -----------------------------------------------------------
     for _ in range(args.warmup):
-        st, nwp, status = guarded("resident", plan)
+        st, wps, status = guarded("resident", plan)
     reached = dev.count_reached()
     assert reached >= 0.90 * n * n, "goal is walled in: only %.3f of the map reached" % (
         reached / float(n * n))
@@ -460,7 +475,7 @@ def headline_plan4096(args, D, pkg, affinity):
     kernel_ms, tiles, updates, outers, written = [], [], [], [], []
     dev.event_record(0)
     for _ in range(args.steps):
-        st, nwp, status = guarded("resident", plan)
+        st, wps, status = guarded("resident", plan)
         kernel_ms.append(st["kernel_ms"])
         tiles.append(st["tile_activations"])
         updates.append(st["cell_updates"])
@@ -471,6 +486,14 @@ def headline_plan4096(args, D, pkg, affinity):
     launches = dev.launches - launches0
     D.barrier()
     clocks = sampler.stop() if rank == 0 else None
+    nwp = len(wps)
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        stride = 1
+        while ((n + stride - 1) // stride) ** 2 * 8 > 48 << 20:
+            stride += 1
+        T = dev.download_total_cost(xform=pkg.cuda_api.XFORM_INF_TO_MINUS1)
+        outputs = {"total_cost": np.ascontiguousarray(T[::stride, ::stride]), "path": wps}
 
     # ---- end-to-end, C ABI: host buffers in, host matrix out, every step ----------------
     cost_host = torch.empty((n, n), dtype=torch.float64).pin_memory()
@@ -643,7 +666,13 @@ def headline_plan4096(args, D, pkg, affinity):
         "plans_run_again_after_a_solver_error": retries["resident"],
         "clocks": clocks,
     }
-    return line, (elev, terr, lut, slopes, locs)
+    return line, (elev, terr, lut, slopes, locs), outputs
+
+
+def dump_outputs(out_dir, outputs):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def stencil_leg(args, D, pkg):
@@ -947,7 +976,9 @@ def run_b200(args):
         res = headline_plan4096(args, D, pkg, affinity)
         dog.leave()
         if D.rank == 0:
-            line, maps = res
+            line, maps, outputs = res
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
             line["stencils"] = stencil_leg(args, D, pkg)
             if not args.no_cpu_baseline and D.world == 1:
                 line["cpu_baseline"] = cpu_baseline_leg(pkg, *maps, args.size)

@@ -33,8 +33,10 @@ def build(ref=True, port=True):
     targets = []
     if port:
         targets.append("port")
-    if ref and os.path.isdir("/root/reference/src"):
-        targets.append("ref")
+    # the unmodified reference sources: /root/reference unless DYMU_REFERENCE names another checkout
+    reference = os.environ.get("DYMU_REFERENCE", "/root/reference")
+    if ref and os.path.isdir(os.path.join(reference, "src")):
+        targets += ["ref", "REFERENCE=" + os.path.abspath(reference)]
     if targets:
         subprocess.run(["make", "-C", HERE] + targets, check=True, stdout=subprocess.DEVNULL)
 
@@ -209,10 +211,30 @@ class Port:
         p = self._l.orc_plane(self._h, self.PLANES[name])
         np.ctypeslib.as_array(p, shape=(self.ny, self.nx))[...] = values
 
+    # DYMU_NODE_* of include/dymu_planner_c.h (fields 1-6 pinned against the reference's taps by
+    # tests/test_golden_cpu.py)
+    NODE_FIELDS = ("elevation", "slope", "raw_cost", "cost", "isObstacle", "state", "hasLocalMap",
+                   "terrain", "total_cost")
+
+    def node_field(self, field):
+        return self.plane(self.NODE_FIELDS[field]).astype(np.float64)
+
     def getTotalCostMatrix(self):
         T = self.plane("total_cost")
         T[np.isinf(T)] = -1.0
         return T
+
+    # the flat-buffer calls of include/dymu_planner_c.h as the C view of the reference makes them
+    # (capi/planner_capi.cpp:442-480): by value through setCostMap / getTotalCostMatrix
+    def setCostMapFlat(self, cost_map):
+        return self.setCostMap(cost_map)
+
+    def setTotalCostMatrixTarget(self, out):
+        return True
+
+    def getTotalCostMatrixFlat(self, out):
+        out[...] = self.getTotalCostMatrix()
+        return True
 
     def getGlobalCostMatrix(self):
         c = self.plane("cost") * (2 + self.plane("hazard_density") - self.plane("trafficability"))

@@ -26,6 +26,8 @@ def replay_config1(factory):
     out["state_early"] = (p.node_field(5) if hasattr(p, "node_field")
                           else p.plane("state").astype(np.float64))
     out["cost"] = (p.node_field(3) if hasattr(p, "node_field") else p.plane("cost"))
+    if hasattr(p, "node_field"):
+        out["slope"], out["raw_cost"] = p.node_field(1), p.node_field(2)
     out["path_early"] = p.getPath(si, sj)
     assert p.computeEntireTotalCostMap()
     out["total_cost_full"] = p.getTotalCostMatrix()
@@ -46,4 +48,6 @@ def replay_repair(factory, approach, name):
     out = dict(path=path, repaired=repaired, traj=traj, risk=p.getRiskMatrix(c[0], c[1]),
                deviation=p.getDeviationMatrix(c[0], c[1]), hazard=p.getHazardDensityMatrix(),
                traff=p.getTrafficabilityMatrix(), reconnecting_index=p.getReconnectingIndex())
+    if hasattr(p, "node_field"):
+        out["has_local"] = p.node_field(6)
     return g, out

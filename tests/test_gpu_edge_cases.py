@@ -1,5 +1,5 @@
-"""Edge cases of the class interface, each run on the compiled unmodified reference and on the
-B200 drop-in with identical calls."""
+"""Edge cases of the class interface, each run on the reference (tests/conftest.py::ref_planner) and
+on the B200 drop-in with identical calls."""
 import numpy as np
 import pytest
 
@@ -9,22 +9,22 @@ from conftest import rel_err
 pytestmark = pytest.mark.gpu
 
 
-def _both(pkg, ref_lib, approach=1, nx=64, ny=64, gres=1.0, lres=0.1, offset=(0.0, 0.0)):
+def _both(pkg, ref, approach=1, nx=64, ny=64, gres=1.0, lres=0.1, offset=(0.0, 0.0)):
     out = []
-    for f in (ref_lib.DyMuPathPlanner, pkg.DyMuPathPlanner):
+    for f in (ref, pkg.DyMuPathPlanner):
         p = f(1.0, 1.5, 2.0, approach)
         assert p.initGlobalLayer(gres, lres, nx, ny, offset)
         out.append(p)
     return out
 
 
-def test_non_unit_global_resolution(pkg, ref_lib):
+def test_non_unit_global_resolution(pkg, ref_planner):
     """global_res = 2.5 m: goal/start conversion, C = res*cost, path step res*tau (G.cpp:326-333,
     527, 706)."""
     nx, ny, gres = 90, 70, 2.5
     cost = pkg.synthetic.smooth_cost_map(ny, nx, seed=3)
     res = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny, gres=gres, lres=0.25):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny, gres=gres, lres=0.25):
         assert p.setCostMap(cost)
         ob = sc.obstacle_plane(p)
         gi, gj = pkg.synthetic.free_interior_cell_near(ob, 70, 50)
@@ -39,10 +39,10 @@ def test_non_unit_global_resolution(pkg, ref_lib):
 
 
 @pytest.mark.parametrize("nx,ny", [(5, 7), (33, 31), (32, 32), (65, 3 + 32)])
-def test_small_and_ragged_grids(pkg, ref_lib, nx, ny):
+def test_small_and_ragged_grids(pkg, ref_planner, nx, ny):
     cost = 1.0 + np.arange(nx * ny, dtype=np.float64).reshape(ny, nx) % 7 * 0.25
     res = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny):
         assert p.setCostMap(cost)
         assert p.setGoal(nx // 2, ny // 2)
         assert p.computeEntireTotalCostMap()
@@ -51,11 +51,11 @@ def test_small_and_ragged_grids(pkg, ref_lib, nx, ny):
     assert rel_err(res[1], res[0]) <= 1e-9
 
 
-def test_replanning_with_a_new_goal_resets_the_map(pkg, ref_lib):
+def test_replanning_with_a_new_goal_resets_the_map(pkg, ref_planner):
     nx = ny = 96
     cost = pkg.synthetic.smooth_cost_map(ny, nx, seed=12)
     res = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny):
         assert p.setCostMap(cost)
         ob = sc.obstacle_plane(p)
         g1 = pkg.synthetic.free_interior_cell_near(ob, 20, 20)
@@ -69,12 +69,12 @@ def test_replanning_with_a_new_goal_resets_the_map(pkg, ref_lib):
         assert rel_err(res[1][k], res[0][k]) <= 1e-9
 
 
-def test_walled_in_start_is_unreachable(pkg, ref_lib):
+def test_walled_in_start_is_unreachable(pkg, ref_planner):
     """computeTotalCostMap returns false when the wave cannot close the start (G.cpp:399-403)."""
     nx = ny = 64
     cost = np.ones((ny, nx))
     cost[20:41, 20] = cost[20:41, 40] = cost[20, 20:41] = cost[40, 20:41] = 0.0   # closed box
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny):
         assert p.setCostMap(cost)
         assert p.setGoal(10.0, 10.0)
         assert not p.computeTotalCostMap(30.0, 30.0)   # inside the box
@@ -83,11 +83,11 @@ def test_walled_in_start_is_unreachable(pkg, ref_lib):
         assert np.all(T[22:39, 22:39] == -1.0)
 
 
-def test_frame_without_obstacles_and_frame_partly_outside(pkg, ref_lib):
+def test_frame_without_obstacles_and_frame_partly_outside(pkg, ref_planner):
     nx = ny = 80
     syn = pkg.synthetic
     res = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny):
         g = sc.global_scenario(p, syn, nx, ny, seed=4, entire=True, goal_frac=(0.8, 0.8),
                                start_frac=(0.1, 0.1))
         path = g["path"]
@@ -108,12 +108,12 @@ def test_frame_without_obstacles_and_frame_partly_outside(pkg, ref_lib):
 
 
 @pytest.mark.parametrize("approach", [1, 0])
-def test_two_consecutive_frames(pkg, ref_lib, approach):
+def test_two_consecutive_frames(pkg, ref_planner, approach):
     """Obstacles seen first off the path (no repair, expansion deferred: L.cpp:278), then a
     second frame that blocks the path: the deferred obstacles must be dilated too."""
     n, syn = 160, pkg.synthetic
     res = []
-    for p in _both(pkg, ref_lib, approach=approach, nx=n, ny=n):
+    for p in _both(pkg, ref_planner, approach=approach, nx=n, ny=n):
         g = sc.global_scenario(p, syn, n, n, seed=9, entire=True)
         path = g["path"]
         c = path[0, :2]
@@ -133,11 +133,11 @@ def test_two_consecutive_frames(pkg, ref_lib, approach):
         assert np.max(np.abs(a[2][:, :2] - b[2][:, :2])) <= 1e-3
 
 
-def test_total_cost_queries_and_node_views(pkg, ref_lib):
+def test_total_cost_queries_and_node_views(pkg, ref_planner):
     nx = ny = 72
     cost = pkg.synthetic.smooth_cost_map(ny, nx, seed=6)
     vals = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny, offset=(3.0, -2.0)):
+    for p in _both(pkg, ref_planner, nx=nx, ny=ny, offset=(3.0, -2.0)):
         assert p.setCostMap(cost)
         ob = sc.obstacle_plane(p)
         gi, gj = pkg.synthetic.free_interior_cell_near(ob, 50, 50)
@@ -157,7 +157,7 @@ def test_node_level_forwards(pkg, ref_lib):
     elev, terr = pkg.synthetic.mars_dem(ny, nx, seed=7)      # (setCostMap alone leaves the reference's
     lut, slopes, locs = pkg.synthetic.default_lut()          #  elevation uninitialised, H.hpp:95)
     out = []
-    for p in _both(pkg, ref_lib, nx=nx, ny=ny):
+    for p in _both(pkg, ref_lib.DyMuPathPlanner, nx=nx, ny=ny):
         assert p.computeCostMap(lut, slopes, locs, elev, terr)
         ob = sc.obstacle_plane(p)
         gi, gj = pkg.synthetic.free_interior_cell_near(ob, 70, 60)

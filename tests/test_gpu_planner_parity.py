@@ -1,6 +1,6 @@
 """GPU parity through the reference-facing class interface: the same call sequence
-(tests/scenarios.py) is issued to the compiled UNMODIFIED reference (oracle/_ref) and to
-the B200 drop-in (libdymu_b200.so -> libdymu_cuda.so).
+(tests/scenarios.py) is issued to the reference (tests/conftest.py::ref_planner: the compiled
+UNMODIFIED reference, or its bit-exact C restatement where that is not built) and to the B200 drop-in (libdymu_b200.so -> libdymu_cuda.so).
 
 Bars (BASELINE.json north_star): obstacle / risk masks and indices bit-exact; total-cost,
 risk and deviation planes <= 1e-9 relative; waypoints <= 1e-3 cell."""
@@ -16,8 +16,8 @@ TOL_PLANE = 1e-9
 TOL_WP = 1e-3
 
 
-def _pair(pkg, ref_lib, approach, nx, ny, **kw):
-    return (sc.make_planner(ref_lib.DyMuPathPlanner, approach, nx, ny, **kw),
+def _pair(pkg, ref, approach, nx, ny, **kw):
+    return (sc.make_planner(ref, approach, nx, ny, **kw),
             sc.make_planner(pkg.DyMuPathPlanner, approach, nx, ny, **kw))
 
 
@@ -26,9 +26,9 @@ def _closed(p):
 
 
 @pytest.mark.parametrize("ny,nx,seed", [(100, 100, 1), (129, 257, 2), (300, 300, 3)])
-def test_entire_total_cost_map_and_path(pkg, ref_lib, ny, nx, seed):
+def test_entire_total_cost_map_and_path(pkg, ref_planner, ny, nx, seed):
     """computeEntireTotalCostMap + getPath (config 1 shape, full solve)."""
-    ref, dut = _pair(pkg, ref_lib, 1, nx, ny)
+    ref, dut = _pair(pkg, ref_planner, 1, nx, ny)
     a = sc.global_scenario(ref, pkg.synthetic, nx, ny, seed, entire=True)
     b = sc.global_scenario(dut, pkg.synthetic, nx, ny, seed, entire=True)
     assert a["ok"] and b["ok"]
@@ -42,12 +42,12 @@ def test_entire_total_cost_map_and_path(pkg, ref_lib, ny, nx, seed):
     assert np.max(np.abs(np.angle(np.exp(1j * (a["path"][:, 3] - b["path"][:, 3]))))) <= 1e-3
 
 
-def test_config1_early_stop(pkg, ref_lib):
+def test_config1_early_stop(pkg, ref_planner):
     """Config 1: 100x100, goal (75,75), start (20,25), computeTotalCostMap(start) + getPath.
     The reference stops once the start node and its 4 neighbours are CLOSED; parity is
     defined on the CLOSED set (SURVEY.md section 7, 'early-stop semantics')."""
     nx = ny = 100
-    ref, dut = _pair(pkg, ref_lib, 1, nx, ny)
+    ref, dut = _pair(pkg, ref_planner, 1, nx, ny)
     a = sc.global_scenario(ref, pkg.synthetic, nx, ny, 1, goal_frac=(0.75, 0.75),
                            start_frac=(0.20, 0.25))
     b = sc.global_scenario(dut, pkg.synthetic, nx, ny, 1, goal_frac=(0.75, 0.75),
@@ -71,7 +71,7 @@ def test_offset_and_locomotion_modes(pkg, ref_lib):
     elev, terr = syn.mars_dem(ny, nx, seed=6)
     lut, slopes, locs = syn.default_lut(n_loc=3)
     out = []
-    for p in _pair(pkg, ref_lib, 0, nx, ny, offset=off):
+    for p in _pair(pkg, ref_lib.DyMuPathPlanner, 0, nx, ny, offset=off):
         assert p.computeCostMap(lut, slopes, locs, elev, terr)
         ob = sc.obstacle_plane(p)
         gi, gj = syn.free_interior_cell_near(ob, 90, 60)
@@ -88,11 +88,11 @@ def test_offset_and_locomotion_modes(pkg, ref_lib):
     assert pa.shape == pb.shape and np.max(np.abs(pa[:, :2] - pb[:, :2])) <= TOL_WP
 
 
-def test_invalid_goals_and_starts(pkg, ref_lib):
+def test_invalid_goals_and_starts(pkg, ref_planner):
     nx = ny = 64
     cost = np.ones((ny, nx))
     cost[30:34, 30:34] = 0.0
-    for p in _pair(pkg, ref_lib, 1, nx, ny):
+    for p in _pair(pkg, ref_planner, 1, nx, ny):
         assert p.setCostMap(cost)
         assert not p.setGoal(-3.0, 5.0)
         assert not p.setGoal(0.0, 10.0)         # border
@@ -108,11 +108,11 @@ def test_invalid_goals_and_starts(pkg, ref_lib):
 
 
 @pytest.mark.parametrize("approach", [1, 0])
-def test_local_repair(pkg, ref_lib, approach):
+def test_local_repair(pkg, ref_planner, approach):
     """Config 2 shape at 200x200: global plan, obstacle frame, computeLocalPlanning."""
     n, syn = 200, pkg.synthetic
     res = []
-    for p in _pair(pkg, ref_lib, approach, n, n):
+    for p in _pair(pkg, ref_planner, approach, n, n):
         g = sc.global_scenario(p, syn, n, n, seed=3, entire=True)
         r = sc.repair_scenario(p, syn, g["path"])
         res.append((g, r, p.node_field(6)))
@@ -132,13 +132,13 @@ def test_local_repair(pkg, ref_lib, approach):
 
 
 @pytest.mark.parametrize("approach", [1, 0])
-def test_config2_1000(pkg, ref_lib, approach):
+def test_config2_1000(pkg, ref_planner, approach):
     """Config 2 at full size (SURVEY.md section 8d): 1000x1000, goal (800,800), start (200,200),
     computeTotalCostMap(start) + getPath, then a 120x120 px frame with an obstacle disc on
     path[10] (+3 random discs, seed 7) -> computeLocalPlanning, SWEEPING and CONSERVATIVE."""
     n, syn = 1000, pkg.synthetic
     res = []
-    for p in _pair(pkg, ref_lib, approach, n, n):
+    for p in _pair(pkg, ref_planner, approach, n, n):
         g = sc.global_scenario(p, syn, n, n, seed=20261018)
         r = sc.repair_scenario(p, syn, g["path"], disc_wp=10)
         res.append((g, r, p.node_field(5), p.node_field(6)))
@@ -169,7 +169,7 @@ def test_cora_loop_rebuilds_cost_map_on_device(pkg, ref_lib):
     rebuilds from the elevation and terrain planes already resident in HBM.  getTerrain
     (G.cpp:941-950) is read from the device terrain plane."""
     nx, ny = 160, 120
-    ref, dut = _pair(pkg, ref_lib, 1, nx, ny)
+    ref, dut = _pair(pkg, ref_lib.DyMuPathPlanner, 1, nx, ny)
     a = sc.global_scenario(ref, pkg.synthetic, nx, ny, 4, entire=True)
     b = sc.global_scenario(dut, pkg.synthetic, nx, ny, 4, entire=True)
     # the transformed read-backs above reuse the staging plane the terrain map was uploaded
@@ -196,7 +196,7 @@ def test_cora_loop_rebuilds_cost_map_on_device(pkg, ref_lib):
     assert rel_err(Tb, b["T"]) > 1e-6                                      # and it matters
 
 
-def test_streamed_cost_map_and_matrix_delivery(pkg, ref_lib):
+def test_streamed_cost_map_and_matrix_delivery(pkg, ref_planner):
     """The copy-free flow of the drop-in -- setCostMap(const double*, ld) with the upload hidden
     behind the solve, total-cost matrix delivered into a caller buffer while getPath runs --
     against the reference driven through the same flat calls (by-value underneath)."""
@@ -208,7 +208,7 @@ def test_streamed_cost_map_and_matrix_delivery(pkg, ref_lib):
     gi, gj = syn.free_interior_cell_near(ob, 500, 300)
     si, sj = syn.free_interior_cell_near(ob, 60, 70)
     out = []
-    for p in _pair(pkg, ref_lib, 1, nx, ny):
+    for p in _pair(pkg, ref_planner, 1, nx, ny):
         T = np.full((ny, nx), 7.0)
         assert p.setCostMapFlat(cost1)           # no goal yet: plain upload
         assert p.setGoal(gi, gj)
@@ -269,7 +269,7 @@ def _repair_at(p, syn, path, k0, seed):
 
 
 @pytest.mark.parametrize("approach", [1, 0])
-def test_local_window_grows_and_keeps_obstacles(pkg, ref_lib, approach, monkeypatch):
+def test_local_window_grows_and_keeps_obstacles(pkg, ref_planner, approach, monkeypatch):
     """The reference's local layer is unbounded and never forgets (L.cpp:150-156, G.cpp:36).  With a
     device window of only 16 global nodes the first frame does not fit (the window is re-created
     larger), the local wave runs into its border (it is doubled and the march repeated), and a
@@ -278,7 +278,7 @@ def test_local_window_grows_and_keeps_obstacles(pkg, ref_lib, approach, monkeypa
     monkeypatch.setenv("DYMU_LOCAL_WINDOW", "16")
     n, syn = 300, pkg.synthetic
     res = []
-    for p in _pair(pkg, ref_lib, approach, n, n):
+    for p in _pair(pkg, ref_planner, approach, n, n):
         g = sc.global_scenario(p, syn, n, n, seed=5, entire=True)
         r1 = _repair_at(p, syn, g["path"], 0, seed=21)
         path = p.current_path
@@ -303,13 +303,13 @@ def test_local_window_grows_and_keeps_obstacles(pkg, ref_lib, approach, monkeypa
     assert np.max(np.abs(hza - hzb)) <= 1e-12 and np.max(np.abs(tra - trb)) <= 1e-9
 
 
-def test_two_repairs_with_incremental_resolve(pkg, ref_lib):
+def test_two_repairs_with_incremental_resolve(pkg, ref_planner):
     """SURVEY.md section 8 row f2: repair -> trafficability / hazard feedback -> total-cost map
     again -> new path -> second repair.  The reference solves from scratch each time; the drop-in
     re-propagates only the dependency cone of the changed nodes (dymu_solve_incremental)."""
     n, syn = 400, pkg.synthetic
     res = []
-    for p in _pair(pkg, ref_lib, 1, n, n):
+    for p in _pair(pkg, ref_planner, 1, n, n):
         g = sc.global_scenario(p, syn, n, n, seed=9, entire=True)
         r1 = _repair_at(p, syn, g["path"], 0, seed=31)
         assert p.computeEntireTotalCostMap()                   # feedback -> re-solve
