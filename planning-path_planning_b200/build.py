@@ -73,10 +73,6 @@ def build_cuda(force=False, verbose=False, ptxas_v=False):
             extra = ["-Xptxas", "-v"] if ptxas_v else []
             if os.environ.get("DYMU_FIM_PROFILE"):
                 extra.append("-DDYMU_FIM_PROFILE")
-            if os.environ.get("DYMU_FIM_WARPS"):
-                extra.append("-DDYMU_FIM_WARPS=" + os.environ["DYMU_FIM_WARPS"])
-            if os.environ.get("DYMU_FIM_ROUNDS"):
-                extra.append("-DDYMU_FIM_ROUNDS=" + os.environ["DYMU_FIM_ROUNDS"])
             if os.environ.get("DYMU_LOCAL_PROFILE"):
                 extra.append("-DDYMU_LOCAL_PROFILE")
             log += _run([NVCC] + NVCC_FLAGS + extra + ["-c", src, "-o", obj], verbose)

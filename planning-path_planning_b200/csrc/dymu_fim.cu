@@ -34,13 +34,9 @@
 //     reset while the next is filled;
 //   * a solve can be stopped after a bounded number of phases and continued later
 //     (dymu_solve_start / dymu_solve_advance): the lists stay consistent at phase boundaries.
-// Environment switches (read once per context): DYMU_FIM_BAND (band width factor, default
-// 4), DYMU_FIM_INNER (sweep cap per activation, default 64), DYMU_FIM_BUDGET /
-// DYMU_FIM_MIN_SLICE (per-CTA sweep budget per phase, default off), DYMU_FIM_GRID_PER_SM,
-// DYMU_FIM_MAX_OUTER, DYMU_FIM_TRACE (per-phase timeline); read per call: DYMU_STREAM_PHASES
-// (streamed solves cut after n / 2n phases instead of on the copy engine's word), DYMU_EXPORT_CAP
-// (tiles a CTA delivers per phase, default 1); build-time: -DDYMU_FIM_PROFILE
-// (clock64 section profile + DYMU_FIM_CTA_TRACE), -DDYMU_FIM_WARPS=8.
+// Environment switch, read per call: DYMU_STREAM_PHASES (streamed solves cut after n / 2n phases
+// instead of on the copy engine's word).  Build-time: -DDYMU_FIM_PROFILE (clock64 section profile,
+// and the per-phase, per-CTA timeline that DYMU_FIM_CTA_TRACE names a file for).
 // Direct delivery (dymu_set_total_cost_export): the kernel tracks an upper bound per tile and
 // stores a tile into the caller's page-locked matrix once that bound is below every pending key
 // (see Params::tmax); k_deliver_rest stores what is left.  A waiting CTA gives up after eight
@@ -57,16 +53,9 @@ namespace
 template <int TILE> struct Cfg
 {
     static_assert(TILE == 32, "4 x 4 blocks of 8 x 8 cells");
-#ifndef DYMU_FIM_ROUNDS
-#define DYMU_FIM_ROUNDS 6  // red-black rounds per block visit (an unchanged block stops early)
-#endif
-#ifndef DYMU_FIM_WARPS
-#define DYMU_FIM_WARPS 16
-#endif
-    static constexpr int WARPS = DYMU_FIM_WARPS;  // 16: one block per warp, 8: two blocks per warp
-    static_assert(WARPS == 16 || WARPS == 8, "warps per tile");
+    static constexpr int ROUNDS = 6;  // red-black rounds per block visit (an unchanged block stops early)
+    static constexpr int WARPS = 16;  // one 8 x 8 block per warp
     static constexpr int THREADS = 32 * WARPS;
-    static constexpr int NB = 16 / WARPS;         // blocks per warp: block b = warp + h * WARPS
     static constexpr int BX = TILE / 8;       // 4 x 4 blocks of 8 x 8 cells, block w <-> warp w
     static constexpr int BY = TILE / 8;
     // row pitch of the shared arrays in doubles.  A half-warp (what one 64-bit shared-memory
@@ -75,7 +64,8 @@ template <int TILE> struct Cfg
     // banks apart and the four groups of alternate columns fall into disjoint banks
     static constexpr int PITCH = TILE + 4;
     static constexpr int CPT = TILE * TILE / THREADS;  // cells per thread in load/store = 2
-    static constexpr int MIN_CTAS = 32 / WARPS;   // 1024 threads per SM either way
+    static constexpr int MIN_CTAS = 2;  // 1024 threads per SM: caps a thread at 64 registers
+    static constexpr int SWEEP_CAP = 2 * TILE;  // sweeps per activation; the rest resumes next phase
     static constexpr size_t SMEM = sizeof(double) * ((TILE + 2) * PITCH + TILE * PITCH);
 };
 
@@ -102,14 +92,11 @@ struct Params
     unsigned long long* key2;
     unsigned long long* gmin;   // [3] minimum key over each list
     uint32_t* dsave;            // per tile: dirty-block mask left over when the sweep cap hit
-    unsigned long long* trace;  // optional: per phase {globaltimer ns, active tiles}, or nullptr
-    uint32_t trace_cap;
     unsigned long long* cta_trace;  // optional (profile build): per phase x CTA timeline
     uint32_t cta_trace_phases;
     uint32_t* ctrl;
     unsigned long long* stats;
-    int inner_cap, max_outer;
-    int phase_budget, min_slice;  // sweeps a CTA may spend per phase; smallest slice worth a tile load
+    int max_outer;
     int outer0;                 // rotation of the three lists at entry (phase-bounded solves)
     double band;                // tiles with key > min key + band wait (inf = plain FIM)
     // direct delivery (MODE 0, one problem).  tmax[tile]: bit pattern of an upper bound of the tile's
@@ -121,7 +108,6 @@ struct Params
     size_t xld;
     uint32_t xnx, xny;          // logical size (the plane is padded to whole tiles)
     int xminus1;                // +inf is delivered as -1 (getTotalCostMatrix, G.cpp:799-811)
-    uint32_t xcap;              // tiles one CTA delivers per phase at most (<= 64)
     const uint32_t* stop_flag;  // leave after the phase in which *stop_flag >= stop_value (nullptr: never)
     uint32_t stop_value;
 };
@@ -301,14 +287,14 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
     __shared__ uint32_t s_tile;
     __shared__ unsigned long long s_emin[5];  // min changed value per edge [0..3], overall [4]
     __shared__ uint32_t s_tmax;                // high word (rounded up) of the largest passable value
-    __shared__ uint32_t s_xn, s_xlist[64];     // tiles this CTA delivers in the current phase
+    __shared__ uint32_t s_xtile;               // the tile this CTA delivers in the current phase
     __shared__ uint32_t s_xorder;              // its order of arrival at the barrier
     __shared__ uint32_t s_bar_ok;              // grid barrier: 0 when the grid is being abandoned
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t tiles_per_prob = p.ntx * p.nty;
-    // ---- per-thread constants of the sweep.  Warp w owns the 8x8 block(s) b = w + h * WARPS
-    // (bx = b & 3, by = b >> 2); lane (lx, ly) owns the two cells (lx, 2 ly) and (lx, 2 ly + 1) of
+    // ---- per-thread constants of the sweep.  Warp w owns the 8x8 block w
+    // (bx = w & 3, by = w >> 2); lane (lx, ly) owns the two cells (lx, 2 ly) and (lx, 2 ly + 1) of
     // it, one of each colour of the checkerboard (x + y even = red).  A block visit relaxes the
     // red cells of the block first and the black ones after a __syncwarp, so the black cells see
     // this very visit's red values: information moves two cells per sweep instead of one
@@ -320,32 +306,27 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
     // The masks live in shared memory: kept in registers the compiler re-derives them from the
     // thread index in every sweep (64-register cap), which costs more issue slots than one load.
     constexpr int c_off = (TILE + 1) * P - 1;  // from a cell of Ts to the same cell of Cs
-    __shared__ uint2 s_wake[K::NB][K::THREADS];
-    double* cell1[K::NB];   // the lane's red cell
+    __shared__ uint2 s_wake[K::THREADS];
+    double* cell1;          // the lane's red cell
     int to_second;          // offset (doubles) from the red to the black cell: +P or -P
-    uint32_t my_bit[K::NB];
+    uint32_t my_bit;
     {
         const int lx = lane & 7, ly = lane >> 3;
         const bool upper_is_red = (lx & 1) == 0;  // rows 2 ly (upper) and 2 ly + 1 (lower)
         to_second = upper_is_red ? P : -P;
         asm volatile("" : "+r"(to_second));
-#pragma unroll
-        for (int h = 0; h < K::NB; ++h)
-        {
-            const int b = warp + h * K::WARPS;
-            const int bx = b & 3, by = b >> 2;
-            // opaque offset: otherwise it is re-derived from the thread index in every sweep
-            int off = (by * 8 + 2 * ly + (upper_is_red ? 0 : 1) + 1) * P + bx * 8 + lx + 1;
-            asm volatile("" : "+r"(off));
-            cell1[h] = Ts + off;
-            my_bit[h] = 1u << b;
-            const uint32_t bitL = bx > 0 ? my_bit[h] >> 1 : 0x40000u, bitR = bx < K::BX - 1 ? my_bit[h] << 1 : 0x80000u;
-            const uint32_t bitU = by > 0 ? my_bit[h] >> 4 : 0x10000u, bitD = by < K::BY - 1 ? my_bit[h] << 4 : 0x20000u;
-            const uint32_t side = (lx == 0 ? bitL : 0u) | (lx == 7 ? bitR : 0u);
-            const uint32_t w_upper = my_bit[h] | side | (ly == 0 ? bitU : 0u);
-            const uint32_t w_lower = my_bit[h] | side | (ly == 3 ? bitD : 0u);
-            s_wake[h][tid] = upper_is_red ? make_uint2(w_upper, w_lower) : make_uint2(w_lower, w_upper);
-        }
+        const int bx = warp & 3, by = warp >> 2;
+        // opaque offset: otherwise it is re-derived from the thread index in every sweep
+        int off = (by * 8 + 2 * ly + (upper_is_red ? 0 : 1) + 1) * P + bx * 8 + lx + 1;
+        asm volatile("" : "+r"(off));
+        cell1 = Ts + off;
+        my_bit = 1u << warp;
+        const uint32_t bitL = bx > 0 ? my_bit >> 1 : 0x40000u, bitR = bx < K::BX - 1 ? my_bit << 1 : 0x80000u;
+        const uint32_t bitU = by > 0 ? my_bit >> 4 : 0x10000u, bitD = by < K::BY - 1 ? my_bit << 4 : 0x20000u;
+        const uint32_t side = (lx == 0 ? bitL : 0u) | (lx == 7 ? bitR : 0u);
+        const uint32_t w_upper = my_bit | side | (ly == 0 ? bitU : 0u);
+        const uint32_t w_lower = my_bit | side | (ly == 3 ? bitD : 0u);
+        s_wake[tid] = upper_is_red ? make_uint2(w_upper, w_lower) : make_uint2(w_lower, w_upper);
     }
     auto sel3 = [](uint32_t* a, uint32_t* b, uint32_t* c, int k) { return k == 0 ? a : (k == 1 ? b : c); };
     auto sel3k = [](unsigned long long* a, unsigned long long* b, unsigned long long* c, int k) {
@@ -385,13 +366,6 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
     {
         const int cur = outer % 3, nxt = (outer + 1) % 3, old = (outer + 2) % 3;
         const uint32_t n_active = ld_volatile_u32(&p.ctrl[cur]);
-        if (p.trace && blockIdx.x == 0 && tid == 0 && (uint32_t)outer < p.trace_cap)
-        {
-            unsigned long long t;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-            p.trace[2 * outer] = t;
-            p.trace[2 * outer + 1] = n_active;
-        }
         if (n_active == 0)
         {
             converged = true;
@@ -426,11 +400,6 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
             if (gm != kNoKey && lim < DYMU_INF) limit = key_of(lim);
         }
 
-        // A phase lasts as long as its busiest CTA.  Every CTA therefore gets a sweep budget per
-        // phase: a tile taken late in the phase is relaxed only for what is left of it (and
-        // resumes from its saved dirty mask next phase), and once the budget is gone the CTA
-        // hands the tiles it still draws to the next phase untouched.
-        int budget = p.phase_budget;
         bool first_fetch = true;
         for (;;)
         {
@@ -457,7 +426,7 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
                     if (idx >= n_active) break;
                     const uint32_t cand = ld_volatile_u32(&list_cur[idx]);
                     const unsigned long long k = ld_volatile_u64(&key_cur[cand]);
-                    if (k <= limit && budget >= p.min_slice)
+                    if (k <= limit)
                     {
                         t = cand;
                         break;
@@ -562,56 +531,45 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
 #endif
 
             // ---- relax in shared memory.  Warp w owns the 8x8 block w (bx = w & 3, by = w >> 2);
-            // lane (lx, ly) owns the cells (lx, ly) and (lx, ly + 4) of it, whose two update
-            // chains are independent and interleave in the in-order issue stream.  A sweep is
+            // lane (lx, ly) owns one red and one black cell of it (see above).  A sweep is
             // therefore one visit per warp, whatever the number of dirty blocks.
             int it = 0;
             uint32_t visits = 0;
             uint32_t m = s_m0;
             uint32_t edges_acc = 0;  // warp-uniform: tile edges this warp's block changed (bits 0..3)
-            const int cap = min(p.inner_cap, budget);
-            double cA[K::NB], cB[K::NB], qA[K::NB], qB[K::NB];
-#pragma unroll
-            for (int h = 0; h < K::NB; ++h)
-            {
-                cA[h] = cell1[h][c_off];
-                cB[h] = cell1[h][to_second + c_off];
-                qA[h] = 2 * (cA[h] * cA[h]);
-                qB[h] = 2 * (cB[h] * cB[h]);
-            }
-            // one sweep: relax the dirty blocks listed in m; returns the next dirty set
+            const double cA = cell1[c_off], cB = cell1[to_second + c_off];
+            const double qA = 2 * (cA * cA), qB = 2 * (cB * cB);
+            // one sweep: relax the warp's block if m lists it dirty; returns the next dirty set
             auto sweep = [&](uint32_t* post) -> uint32_t {
                 uint32_t contrib = 0;
-#pragma unroll
-                for (int h = 0; h < K::NB; ++h)
+                if (m & my_bit)
                 {
-                    if (!(m & my_bit[h])) continue;
-                    double* a = cell1[h];
+                    double* a = cell1;
                     double* b = a + to_second;
                     // requested with the cell values and pinned here: left to the compiler the
                     // load sinks below the update and its latency lands on the chain
-                    uint2 wake = s_wake[h][tid];
+                    uint2 wake = s_wake[tid];
                     asm volatile("" : "+r"(wake.x), "+r"(wake.y));
                     uint32_t woke = 0;
 #pragma unroll
-                    for (int round = 0; round < DYMU_FIM_ROUNDS; ++round)
+                    for (int round = 0; round < K::ROUNDS; ++round)
                     {
                         // red cells of the block ...
                         double tA = a[0];
                         const double lA = a[-1], rA = a[1], uA = a[-P], dA = a[P];
                         asm volatile("" : "+d"(tA));
                         double nA, nB;
-                        const bool chA = relax<MODE>(tA, lA, rA, uA, dA, cA[h], qA[h], nA);
+                        const bool chA = relax<MODE>(tA, lA, rA, uA, dA, cA, qA, nA);
                         if (chA) a[0] = nA;
                         __syncwarp();
                         // ... then the black ones, on the red values just stored
                         const double tB = b[0];
                         const double lB = b[-1], rB = b[1], uB = b[-P], dB = b[P];
-                        const bool chB = relax<MODE>(tB, lB, rB, uB, dB, cB[h], qB[h], nB);
+                        const bool chB = relax<MODE>(tB, lB, rB, uB, dB, cB, qB, nB);
                         if (chB) b[0] = nB;
                         woke |= (chA ? wake.x : 0u) | (chB ? wake.y : 0u);
                         visits += 2;
-                        if (round + 1 < DYMU_FIM_ROUNDS)
+                        if (round + 1 < K::ROUNDS)
                         {
                             // another round only pays while the block is still changing
                             if (!__any_sync(0xffffffffu, chA || chB)) break;
@@ -619,7 +577,7 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
                     }
                     // one warp reduction tells which blocks (bits 0..15) and which tile edges
                     // (bits 16..19) saw a change
-                    contrib |= __reduce_or_sync(0xffffffffu, woke);
+                    contrib = __reduce_or_sync(0xffffffffu, woke);
                 }
                 edges_acc |= contrib >> 16;
                 if (lane == 0) post[warp] = contrib & 0xffffu;
@@ -629,9 +587,9 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
             };
             for (;;)
             {
-                if (m == 0 || it >= cap) break;
+                if (m == 0 || it >= K::SWEEP_CAP) break;
                 m = sweep(s_post[0]);
-                if (m == 0 || it >= cap) break;
+                if (m == 0 || it >= K::SWEEP_CAP) break;
                 m = sweep(s_post[1]);
             }
             if (edges_acc && lane == 0) smem_or(&edge_mask, edges_acc);
@@ -732,7 +690,6 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
             }
             n_tiles++;
             n_inner += (unsigned long long)it;
-            budget -= it;
             PC_MARK(pc_store)
 #ifdef DYMU_FIM_PROFILE
             if (tid == 0) { GT(tl_store) tl_tiles++; }
@@ -760,34 +717,34 @@ __global__ void __launch_bounds__(Cfg<TILE>::THREADS, Cfg<TILE>::MIN_CTAS) k_fim
         {
             // Between arriving at the barrier and leaving it, the CTAs that arrive in the first half
             // -- they would only wait -- look through the tile bounds (a share of the array each,
-            // by order of arrival) and deliver the tiles the front has left behind.  The CTAs the
-            // others are waiting for skip this, so a phase is not made longer.
+            // by order of arrival) and deliver one of the tiles the front has left behind.  The CTAs
+            // the others are waiting for skip this, so a phase is not made longer.
+            // One tile per CTA and phase keeps the delivery inside the time an early CTA would wait at
+            // the barrier anyway (4096^2: solve 7.82 ms without, 7.90 ms with; 8.28 ms at 64 per phase);
+            // the half of the grid that delivers still moves 148 tiles per phase, twice what finishes.
             // the smallest key that was pending when this phase began: every value below it is final.
             // Read BEFORE arriving -- nothing writes gmin[cur] during its own phase, but once this CTA
             // has arrived the others may run ahead and recycle that slot for the phase after next.
             const unsigned long long gm = ld_volatile_u64(&p.gmin[cur]);
             grid_barrier_arrive(&p.ctrl[6], phase, &s_xorder);
-            if (tid == 0) s_xn = 0;
+            if (tid == 0) s_xtile = 0xffffffffu;
             __syncthreads();
             const uint32_t order = s_xorder, sharers = max(gridDim.x / 2u, 1u);
             if (order < sharers)
             {
                 const uint32_t per = (tiles_per_prob + sharers - 1) / sharers;
                 const uint32_t t_end = min((order + 1) * per, tiles_per_prob);
+                // the first final tile found is claimed; the others are found again next phase
                 for (uint32_t t = order * per + tid; t < t_end; t += K::THREADS)
-                    if (ld_volatile_u64(&p.tmax[t]) < gm)
-                    {
-                        const uint32_t q = atomicAdd(&s_xn, 1u);
-                        if (q < p.xcap)  // the rest is found again next phase
-                        {
-                            s_xlist[q] = t;
-                            p.tmax[t] = kExported;
-                        }
-                    }
+                    if (ld_volatile_u64(&p.tmax[t]) < gm && atomicCAS(&s_xtile, 0xffffffffu, t) == 0xffffffffu)
+                        p.tmax[t] = kExported;
                 __syncthreads();
-                const uint32_t n = min(s_xn, p.xcap);
-                for (uint32_t q = 0; q < n; ++q) deliver_tile(s_xlist[q]);
-                if (tid == 0 && n) atomicAdd(&p.stats[7], (unsigned long long)n);
+                const uint32_t xt = s_xtile;
+                if (xt != 0xffffffffu)
+                {
+                    deliver_tile(xt);
+                    if (tid == 0) atomicAdd(&p.stats[7], 1ull);
+                }
             }
             if (!grid_barrier_wait(&p.ctrl[6], phase, &p.stats[14], &s_bar_ok)) break;
         }
@@ -968,7 +925,6 @@ template <int TILE, int MODE> int launch_fim(dymu_ctx* ctx, Params& prm, size_t 
     DYMU_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(
                            &per_sm, k_fim<TILE, MODE>, Cfg<TILE>::THREADS, Cfg<TILE>::SMEM));
     if (per_sm < 1) DYMU_FAIL(ctx, DYMU_ERR_CUDA, "FIM kernel does not fit on an SM");
-    if (ctx->fim_grid_per_sm > 0 && ctx->fim_grid_per_sm < per_sm) per_sm = ctx->fim_grid_per_sm;
     size_t grid = (size_t)per_sm * ctx->sm_count;
     if (grid > total_tiles) grid = total_tiles;
     if (grid < 1) grid = 1;
@@ -1031,21 +987,7 @@ int dymu_internal_fim_configure(dymu_ctx* ctx)
     int dev_coop = 0;
     DYMU_CUDA_TRY(ctx, cudaDeviceGetAttribute(&dev_coop, cudaDevAttrCooperativeLaunch, ctx->device));
     if (!dev_coop) DYMU_FAIL(ctx, DYMU_ERR_NODEVICE, "device lacks cooperative launch");
-    ctx->fim_inner_cap = (int)ctx->tile * 2;
-    if (const char* e = getenv("DYMU_FIM_INNER"))
-        if (atoi(e) > 0) ctx->fim_inner_cap = atoi(e);
-    ctx->fim_phase_budget = 0;  // sweeps per CTA per phase; 0 = unlimited
-    if (const char* e = getenv("DYMU_FIM_BUDGET")) ctx->fim_phase_budget = atoi(e);
-    ctx->fim_min_slice = 12;
-    if (const char* e = getenv("DYMU_FIM_MIN_SLICE"))
-        if (atoi(e) > 0) ctx->fim_min_slice = atoi(e);
-    ctx->fim_grid_per_sm = 0;  // 0 = as many CTAs per SM as fit
-    if (const char* e = getenv("DYMU_FIM_GRID_PER_SM"))
-        if (atoi(e) > 0) ctx->fim_grid_per_sm = atoi(e);
-    ctx->fim_max_outer = 0;  // derived per launch
-    ctx->fim_band_factor = 4.0;  // band = factor * tile * mean(C_eff); <= 0 disables banding
-    if (const char* e = getenv("DYMU_FIM_BAND")) ctx->fim_band_factor = atof(e);
-    ctx->fim_band = 1.0 / 0.0;
+    ctx->fim_band = 1.0 / 0.0;  // until C_eff is first computed
     return DYMU_OK;
 }
 
@@ -1124,8 +1066,6 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
     prm.key0 = w->key[0]; prm.key1 = w->key[1]; prm.key2 = w->key[2];
     prm.gmin = w->gmin;
     prm.dsave = w->dsave;
-    prm.trace = nullptr;
-    prm.trace_cap = 0;
     prm.cta_trace = nullptr;
     prm.cta_trace_phases = 0;
     unsigned long long* d_cta_trace = nullptr;
@@ -1141,16 +1081,6 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
         prm.cta_trace_phases = cta_trace_phases;
     }
 #endif
-    const char* trace_path = getenv("DYMU_FIM_TRACE");
-    unsigned long long* d_trace = nullptr;
-    const uint32_t trace_cap = 8192;
-    if (trace_path && L.mode == 0)
-    {
-        DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&d_trace, trace_cap * 16));
-        DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d_trace, 0, trace_cap * 16, ctx->stream));
-        prm.trace = d_trace;
-        prm.trace_cap = trace_cap;
-    }
     prm.ctrl = w->ctrl;
     prm.stats = w->stats;
     prm.stop_flag = L.stop_flag;
@@ -1161,12 +1091,6 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
     prm.xnx = ctx->nx;
     prm.xny = ctx->ny;
     prm.xminus1 = ctx->export_xform == DYMU_XFORM_INF_TO_MINUS1;
-    // One tile per CTA and phase keeps the delivery inside the time an early CTA would wait at the
-    // barrier anyway (4096^2: solve 7.82 ms without, 7.90 ms with; 8.28 ms at 64 per phase); the
-    // half of the grid that delivers still moves 148 tiles per phase, twice what finishes.
-    prm.xcap = 1;
-    if (const char* e = getenv("DYMU_EXPORT_CAP"))
-        if (atoi(e) > 0 && atoi(e) <= 64) prm.xcap = (uint32_t)atoi(e);
     if (L.mode == 0 && L.nprob == 1 && L.T == ctx->T && ctx->tile_tmax && (L.track_final || L.export_now))
     {
         prm.tmax = ctx->tile_tmax;
@@ -1177,14 +1101,9 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
         }
     }
     prm.band = L.band;
-    prm.inner_cap = ctx->fim_inner_cap;
-    prm.phase_budget = ctx->fim_phase_budget > 0 ? ctx->fim_phase_budget : 1 << 30;
-    prm.min_slice = ctx->fim_min_slice;
     // a wave needs at most ~(ntx+nty) tile hops in free space; obstacles lengthen the
     // geodesic, so leave two orders of magnitude of head room before reporting NOCONV
     prm.max_outer = 64 * (int)(L.ntx + L.nty) + 4096;
-    if (const char* e = getenv("DYMU_FIM_MAX_OUTER"))
-        if (atoi(e) > 0) prm.max_outer = atoi(e);
     if (L.max_phases > 0) prm.max_outer = (int)L.max_phases;
     const bool bounded = L.max_phases > 0 || L.stop_flag;
     prm.outer0 = w->rot;
@@ -1234,19 +1153,6 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
         }
         free(hb);
         cudaFree(d_cta_trace);
-    }
-    if (d_trace)
-    {
-        unsigned long long* ht = (unsigned long long*)malloc(trace_cap * 16);
-        cudaMemcpy(ht, d_trace, trace_cap * 16, cudaMemcpyDeviceToHost);
-        if (FILE* f = fopen(trace_path, "w"))
-        {
-            for (uint32_t k = 0; k < trace_cap && ht[2 * k]; ++k)
-                fprintf(f, "%u %llu %llu\n", k, ht[2 * k] - ht[0], ht[2 * k + 1]);
-            fclose(f);
-        }
-        free(ht);
-        cudaFree(d_trace);
     }
     if (stats)
     {

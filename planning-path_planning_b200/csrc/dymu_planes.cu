@@ -10,6 +10,9 @@
 namespace
 {
 constexpr int kThreads = 256;
+// band width of the tile scheduler (dymu_fim.cu) in units of tile * mean(C_eff): a few tile
+// crossings worth of total cost (DESIGN.md section 5: flat around 4 over a grid of 24 settings)
+constexpr double kBandFactor = 4.0;
 
 inline int stream_grid(const dymu_ctx* ctx, size_t work_items, int per_thread = 1)
 {
@@ -991,7 +994,7 @@ int dymu_internal_settle_upload(dymu_ctx* ctx)
 int dymu_internal_band_from_rows(dymu_ctx* ctx, uint32_t j0, uint32_t j1)
 {
     ctx->fim_band = 1.0 / 0.0;
-    if (!(ctx->fim_band_factor > 0) || j0 >= j1 || j1 > ctx->rows) return DYMU_OK;
+    if (j0 >= j1 || j1 > ctx->rows) return DYMU_OK;
     const size_t n = (size_t)ctx->pitch * (j1 - j0);
     DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
     double* d = (double*)ctx->d_scratch;
@@ -1002,7 +1005,7 @@ int dymu_internal_band_from_rows(dymu_ctx* ctx, uint32_t j0, uint32_t j1)
     double h[2] = {0, 0};
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (h[1] > 0) ctx->fim_band = ctx->fim_band_factor * (double)ctx->tile * (h[0] / h[1]);
+    if (h[1] > 0) ctx->fim_band = kBandFactor * (double)ctx->tile * (h[0] / h[1]);
     return DYMU_OK;
 }
 
@@ -1012,28 +1015,19 @@ int dymu_internal_refresh_ceff(dymu_ctx* ctx)
     size_t n = (size_t)ctx->pitch * ctx->rows;
     // the same pass accumulates sum and count of the finite values: the band width of the tile
     // scheduler is a few tile crossings worth of total cost
-    const bool want_band = ctx->fim_band_factor > 0;
-    double* d = nullptr;
-    if (want_band)
-    {
-        DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
-        d = (double*)ctx->d_scratch;
-        DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 16, ctx->stream));
-    }
+    DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
+    double* d = (double*)ctx->d_scratch;
+    DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 16, ctx->stream));
     k_ceff<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->cost, ctx->haz, ctx->traff,
                                                              ctx->obst, ctx->ceff, ctx->gres,
                                                              ctx->pitch, ctx->rows, ctx->nx,
                                                              ctx->ny, d);
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
-    ctx->fim_band = 1.0 / 0.0;
-    if (want_band)
-    {
-        double h[2] = {0, 0};
-        DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
-        DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-        if (h[1] > 0) ctx->fim_band = ctx->fim_band_factor * (double)ctx->tile * (h[0] / h[1]);
-    }
+    double h[2] = {0, 0};
+    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->fim_band = h[1] > 0 ? kBandFactor * (double)ctx->tile * (h[0] / h[1]) : 1.0 / 0.0;
     ctx->ceff_dirty = false;
     return DYMU_OK;
 }
