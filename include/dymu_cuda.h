@@ -149,11 +149,6 @@ int dymu_reserve_slots(dymu_ctx* ctx, uint32_t n_slots);
  * (aggregate numbers are reported in stats[0]). */
 int dymu_solve_total_cost(dymu_ctx* ctx, uint32_t n_goals, const uint32_t* goal_i,
                           const uint32_t* goal_j, dymu_solve_stats* stats);
-/* Continue a solve after total-cost values were lowered from outside (domain
- * decomposition halo rows): re-activates the tiles covering the row ranges
- * [ranges[2k], ranges[2k+1]) of slot 0 and iterates to convergence. */
-int dymu_solve_resume(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges,
-                      dymu_solve_stats* stats);
 /* Phase-bounded variants for pipelined domain decomposition (one GPU per row strip of a grid
  * too large or too slow for one GPU).  The propagation of computeEntireTotalCostMap
  * (G.cpp:443-468) is advanced by at most `max_phases` solver phases per call; the pending work
@@ -163,7 +158,9 @@ int dymu_solve_resume(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges,
  *                       just lowered by dymu_import_rows_min_key; n_ranges may be 0) into the
  *                       pending work with priority `seed_key` (the smallest lowered value) and
  *                       run <= max_phases more.  A strip without the goal starts with
- *                       dymu_reset_total_cost and its first import. */
+ *                       dymu_reset_total_cost and its first import.  When nothing is pending
+ *                       (after a converged solve or dymu_reset_total_cost), the call wakes the
+ *                       tiles of `ranges` on a clean work list. */
 int dymu_solve_start(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, uint32_t max_phases,
                      dymu_solve_stats* stats);
 int dymu_solve_advance(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges, double seed_key,
@@ -202,13 +199,11 @@ int dymu_plan_streamed(dymu_ctx* ctx, const double* cost_host, size_t ld, uint32
 int dymu_reset_total_cost(dymu_ctx* ctx);
 /* Halo exchange for row-strip domain decomposition.  Rows are dense (nx doubles each).
  * `device_ptr` != 0: dst/src is device memory of this GPU, otherwise host memory.
- * import takes the element-wise minimum with the resident rows and reports whether any
- * value decreased. */
+ * import takes the element-wise minimum with the resident rows, reports whether any
+ * value decreased and sets *min_lowered = the smallest value that replaced a larger one
+ * (+inf if none). */
 int dymu_export_rows(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows, double* dst,
                      int device_ptr);
-int dymu_import_rows_min(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
-                         const double* src, int device_ptr, int* changed);
-/* same, and *min_lowered = the smallest value that replaced a larger one (+inf if none) */
 int dymu_import_rows_min_key(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
                              const double* src, int device_ptr, int* changed, double* min_lowered);
 int dymu_count_reached(dymu_ctx* ctx, uint32_t slot, uint64_t* n_finite);

@@ -1354,14 +1354,13 @@ int dymu_solve_start(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, uint32_t m
     return solve_total_cost_impl(ctx, 1, &goal_i, &goal_j, max_phases, stats);
 }
 
-static int solve_resume_impl(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges, bool keep_pending,
-                             double seed_key, uint32_t max_phases, dymu_solve_stats* stats,
-                             bool deliver = false)
+static int solve_resume_impl(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges, double seed_key,
+                             uint32_t max_phases, dymu_solve_stats* stats, bool deliver = false)
 {
     if (!ctx || (!ranges && n_ranges)) return DYMU_ERR_ARG;
     if (!deliver) ctx->export_done = false;
     if (!ctx->have_cost) DYMU_FAIL(ctx, DYMU_ERR_STATE, "no cost map");
-    if (n_ranges == 0 && !(keep_pending && ctx->work.pending))
+    if (n_ranges == 0 && !ctx->work.pending)
     {
         // nothing queued and nothing new: the plane is at its fixed point
         if (stats)
@@ -1405,7 +1404,7 @@ static int solve_resume_impl(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_r
     L.pitch = ctx->pitch; L.rows = ctx->rows; L.ntx = ctx->ntx; L.nty = ctx->nty; L.nprob = 1;
     L.mode = 0; L.tile = (int)ctx->tile; L.work = &ctx->work; L.n_initial = n_rows; L.band = ctx->fim_band;
     L.seed_kind = n_rows ? 1 : 3; L.seed_data = (const uint32_t*)ctx->d_scratch;
-    L.resume = keep_pending;
+    L.resume = true;
     L.max_phases = max_phases;
     L.seed_key = seed_key;
     if (ctx->stream_stop_value)
@@ -1423,19 +1422,12 @@ static int solve_resume_impl(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_r
     return rc;
 }
 
-int dymu_solve_resume(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges, dymu_solve_stats* stats)
-{
-    DYMU_GUARD(ctx);
-    if (!ranges || n_ranges == 0) return DYMU_ERR_ARG;
-    return solve_resume_impl(ctx, ranges, n_ranges, false, 0.0, 0, stats);
-}
-
 int dymu_solve_advance(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_ranges, double seed_key,
                        uint32_t max_phases, dymu_solve_stats* stats)
 {
     DYMU_GUARD(ctx);
     if (max_phases == 0 || !(seed_key >= 0.0)) return DYMU_ERR_ARG;
-    return solve_resume_impl(ctx, ranges, n_ranges, true, seed_key, max_phases, stats);
+    return solve_resume_impl(ctx, ranges, n_ranges, seed_key, max_phases, stats);
 }
 
 int dymu_set_cost_map_begin(dymu_ctx* ctx, const double* cost_host, size_t ld, uint32_t first_row)
@@ -1554,7 +1546,7 @@ static int solve_streamed(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, uint3
         if (!all_there || first_phases)
         {
             ctx->stream_stop_value = first_phases ? 0 : 2;
-            rc = solve_resume_impl(ctx, ranges, n_ranges, true, 0.0, first_phases ? 2 * first_phases : (1u << 20),
+            rc = solve_resume_impl(ctx, ranges, n_ranges, 0.0, first_phases ? 2 * first_phases : (1u << 20),
                                    &part[1]);
             ctx->stream_stop_value = 0;
             n_ranges = 0;
@@ -1581,7 +1573,7 @@ static int solve_streamed(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, uint3
         return DYMU_OK;
     }
     if (n3 || ctx->work.pending)
-        rc = solve_resume_impl(ctx, ranges3, n3, true, 0.0, 0, &part[2], true);
+        rc = solve_resume_impl(ctx, ranges3, n3, 0.0, 0, &part[2], true);
     else
         part[2].converged = 1;
     if (stats)
@@ -1640,10 +1632,11 @@ int dymu_export_rows(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
     return DYMU_OK;
 }
 
-static int import_rows_impl(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows, const double* src,
-                            int device_ptr, int* changed, double* min_lowered)
+int dymu_import_rows_min_key(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
+                             const double* src, int device_ptr, int* changed, double* min_lowered)
 {
-    if (!ctx || !src || !changed || slot >= ctx->n_slots || n_rows == 0
+    DYMU_GUARD(ctx);
+    if (!ctx || !src || !changed || !min_lowered || slot >= ctx->n_slots || n_rows == 0
         || (uint64_t)j0 + n_rows > ctx->ny)
         return DYMU_ERR_ARG;
     DYMU_TRY(dymu_internal_settle_delivery(ctx));
@@ -1674,29 +1667,11 @@ static int import_rows_impl(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t 
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     *changed = (int)(h[0] & 0xffffffffu);
     if (*changed) ctx->solved = ctx->export_done = false;  // the plane moved away from the last solve's fixed point
-    if (min_lowered)
-    {
-        long long bits = (long long)h[1];
-        double v;
-        memcpy(&v, &bits, sizeof(v));
-        *min_lowered = *changed ? v : 1.0 / 0.0;
-    }
+    long long bits = (long long)h[1];
+    double v;
+    memcpy(&v, &bits, sizeof(v));
+    *min_lowered = *changed ? v : 1.0 / 0.0;
     return DYMU_OK;
-}
-
-int dymu_import_rows_min(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
-                         const double* src, int device_ptr, int* changed)
-{
-    DYMU_GUARD(ctx);
-    return import_rows_impl(ctx, slot, j0, n_rows, src, device_ptr, changed, nullptr);
-}
-
-int dymu_import_rows_min_key(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t n_rows,
-                             const double* src, int device_ptr, int* changed, double* min_lowered)
-{
-    DYMU_GUARD(ctx);
-    if (!min_lowered) return DYMU_ERR_ARG;
-    return import_rows_impl(ctx, slot, j0, n_rows, src, device_ptr, changed, min_lowered);
 }
 
 int dymu_stop_threshold(dymu_ctx* ctx, uint32_t slot, uint32_t start_i, uint32_t start_j,

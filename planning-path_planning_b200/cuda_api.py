@@ -84,7 +84,6 @@ _SIG = {
     "dymu_reserve_slots": (C.c_int, [C.c_void_p, C.c_uint32]),
     "dymu_solve_total_cost": (C.c_int, [C.c_void_p, C.c_uint32, _u32p, _u32p,
                                         C.POINTER(SolveStats)]),
-    "dymu_solve_resume": (C.c_int, [C.c_void_p, _u32p, C.c_uint32, C.POINTER(SolveStats)]),
     "dymu_solve_start": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(SolveStats)]),
     "dymu_solve_advance": (C.c_int, [C.c_void_p, _u32p, C.c_uint32, C.c_double, C.c_uint32,
                                      C.POINTER(SolveStats)]),
@@ -92,8 +91,6 @@ _SIG = {
                                      C.POINTER(SolveStats)]),
     "dymu_reset_total_cost": (C.c_int, [C.c_void_p]),
     "dymu_export_rows": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
-    "dymu_import_rows_min": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
-                                       C.c_int, C.POINTER(C.c_int)]),
     "dymu_import_rows_min_key": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
                                            C.c_int, C.POINTER(C.c_int), _dp]),
     "dymu_count_reached": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]),
@@ -303,14 +300,6 @@ class DeviceLayer:
         self._chk(self._l.dymu_solve_incremental(self._h, int(goal[0]), int(goal[1]), C.byref(st), C.byref(inv)))
         return st.as_dict(), (None if inv.value == 2 ** 64 - 1 else int(inv.value))
 
-    def solve_resume(self, ranges):
-        """ranges: iterable of (j0, j1) row ranges whose tiles are re-activated."""
-        r = np.ascontiguousarray(list(ranges), dtype=np.uint32).reshape(-1, 2)
-        st = SolveStats()
-        self._chk(self._l.dymu_solve_resume(self._h, r.ctypes.data_as(_u32p), r.shape[0],
-                                            C.byref(st)))
-        return st.as_dict()
-
     def solve_start(self, goal, max_phases):
         """Seed the goal and run at most max_phases solver phases; stats['converged'] == 0 means
         work is pending on the device (continue with solve_advance)."""
@@ -353,12 +342,6 @@ class DeviceLayer:
     def export_rows(self, j0, n_rows, dst_ptr, device_ptr, slot=0):
         self._chk(self._l.dymu_export_rows(self._h, slot, j0, n_rows, C.c_void_p(dst_ptr),
                                            int(device_ptr)))
-
-    def import_rows_min(self, j0, n_rows, src_ptr, device_ptr, slot=0):
-        ch = C.c_int()
-        self._chk(self._l.dymu_import_rows_min(self._h, slot, j0, n_rows, C.c_void_p(src_ptr),
-                                               int(device_ptr), C.byref(ch)))
-        return bool(ch.value)
 
     def import_rows_min_key(self, j0, n_rows, src_ptr, device_ptr, slot=0):
         """-> (changed, smallest value that replaced a larger one or +inf)."""

@@ -4,18 +4,15 @@ Two cases shard naturally:
 
 * independent goal queries / maps -- ``shard_queries``: block assignment of queries to
   ranks, no data-path collective (each rank holds the read-only cost planes);
-* one very large grid -- row-strip domain decomposition (``strip_rows`` + ``dd_solve``): each
-  rank owns a contiguous band of rows plus one ghost row per interior side.  A rank
-  relaxes its strip to local convergence, then boundary rows are exchanged with the two
-  neighbours (point-to-point) and a 1-word all-reduce decides termination.  Ghost rows
+* one very large grid -- row-strip domain decomposition (``strip_rows`` +
+  ``dd_solve_pipelined``): each rank owns a contiguous band of rows plus one ghost row per
+  interior side.  Every round, a rank advances its strip by a bounded number of solver
+  phases (``dymu_solve_start`` / ``dymu_solve_advance`` keep the pending work on the
+  device), boundary rows are exchanged with the two neighbours (point-to-point) and a
+  1-word all-reduce decides termination.  A neighbour starts as soon as the wave front
+  crosses the cut instead of after the whole strip behind it has converged.  Ghost rows
   carry C_eff = +inf, so they are never updated locally and act as Dirichlet data; values
   only ever decrease, so the iteration converges to the single-grid fixed point.
-
-``dd_solve_pipelined`` is the same decomposition without the "converge, then talk" rhythm:
-every rank advances its strip by a bounded number of solver phases per round
-(``dymu_solve_start`` / ``dymu_solve_advance`` keep the pending work on the device), so a
-neighbour starts as soon as the wave front crosses the cut instead of after the whole strip
-behind it has converged.
 
 The driver is written against two small interfaces so that the very same control flow runs
 on GPUs (``CudaStrip`` + torch.distributed/NCCL) and in the CPU test-suite (a numpy strip
@@ -122,37 +119,15 @@ class CudaStrip:
         self._row = {k: torch.empty(nx, dtype=torch.float64, device=self.device) for k in "tb"}
         self.stats = []
 
-    def start(self, goal_global):
-        """Initial local solve: the rank owning the goal seeds it, the others start at +inf."""
-        gi, gj = goal_global
-        if self.layout.owns(gj):
-            self.stats.append(self.dev.solve_total_cost([(gi, self.layout.local_row(gj))]))
-        else:
-            self.dev.reset_total_cost()
-
     def boundary_rows(self):
         lay = self.layout
         self.dev.export_rows(lay.first_own, 1, self._row["t"].data_ptr(), True)
         self.dev.export_rows(lay.last_own, 1, self._row["b"].data_ptr(), True)
         return self._row["t"], self._row["b"]
 
-    def absorb(self, from_above, from_below):
-        """Min-merges neighbour rows into the ghost rows; returns the row ranges to resume."""
-        lay, ranges = self.layout, []
-        if from_above is not None and self.dev.import_rows_min(0, 1, from_above.data_ptr(), True):
-            ranges.append((0, 2))
-        if from_below is not None and self.dev.import_rows_min(lay.ny_local - 1, 1,
-                                                               from_below.data_ptr(), True):
-            ranges.append((lay.ny_local - 2, lay.ny_local))
-        return ranges
-
-    def resume(self, ranges):
-        self.stats.append(self.dev.solve_resume(ranges))
-
-    # -- phase-bounded protocol (dd_solve_pipelined) ------------------------------------
-    def start_bounded(self, goal_global, phases):
-        """Like start(), but stops after `phases` solver phases.  Returns True while work is
-        pending on the device."""
+    def start(self, goal_global, phases):
+        """Initial local solve of at most `phases` solver phases: the rank owning the goal seeds
+        it, the others start at +inf.  Returns True while work is pending on the device."""
         gi, gj = goal_global
         if self.layout.owns(gj):
             st = self.dev.solve_start((gi, self.layout.local_row(gj)), phases)
@@ -161,9 +136,10 @@ class CudaStrip:
         self.dev.reset_total_cost()
         return False
 
-    def absorb_keyed(self, from_above, from_below):
-        """absorb() that also returns the smallest value a ghost row was lowered to: the
-        priority the re-activated tiles get among the pending ones."""
+    def absorb(self, from_above, from_below):
+        """Min-merges neighbour rows into the ghost rows.  Returns the row ranges to wake and
+        the smallest value a ghost row was lowered to: the priority the woken tiles get among
+        the pending ones."""
         lay, ranges, key = self.layout, [], float("inf")
         if from_above is not None:
             ch, lo = self.dev.import_rows_min_key(0, 1, from_above.data_ptr(), True)
@@ -188,22 +164,6 @@ class CudaStrip:
         return T[lay.first_own:lay.last_own + 1]
 
 
-def dd_solve(strip, comm, goal_global, max_rounds=10000):
-    """Domain-decomposed total-cost solve.  Returns the number of exchange rounds."""
-    strip.start(goal_global)
-    rounds = 0
-    while rounds < max_rounds:
-        top, bottom = strip.boundary_rows()
-        from_above, from_below = comm.exchange(top, bottom)
-        ranges = strip.absorb(from_above, from_below)
-        rounds += 1
-        if not comm.any(bool(ranges)):
-            break
-        if ranges:
-            strip.resume(ranges)
-    return rounds
-
-
 def dd_solve_pipelined(strip, comm, goal_global, phases_per_round=16, max_rounds=1000000):
     """Domain-decomposed solve with bounded work per exchange round: every rank runs at most
     `phases_per_round` solver phases, trades boundary rows, merges what it received into its
@@ -218,12 +178,12 @@ def dd_solve_pipelined(strip, comm, goal_global, phases_per_round=16, max_rounds
         lap[name] += time.perf_counter() - t0
         return out
 
-    pending = timed("advance", strip.start_bounded, goal_global, phases_per_round)
+    pending = timed("advance", strip.start, goal_global, phases_per_round)
     rounds = 0
     while rounds < max_rounds:
         top, bottom = timed("export", strip.boundary_rows)
         from_above, from_below = timed("exchange", comm.exchange, top, bottom)
-        ranges, key = timed("absorb", strip.absorb_keyed, from_above, from_below)
+        ranges, key = timed("absorb", strip.absorb, from_above, from_below)
         rounds += 1
         if not timed("vote", comm.any, bool(ranges) or pending):
             break
@@ -232,12 +192,11 @@ def dd_solve_pipelined(strip, comm, goal_global, phases_per_round=16, max_rounds
     return rounds
 
 
-def dd_solve_lockstep(strips, goal_global, max_rounds=10000):
-    """The same decomposition with all strips in ONE process (k logical shards on one device,
-    or several devices driven by one host thread): rows are handed over directly instead of
+def dd_solve_lockstep(strips, goal_global, phases_per_round=16, max_rounds=1000000):
+    """dd_solve_pipelined with all strips in ONE process (k logical shards on one device, or
+    several devices driven by one host thread): rows are handed over directly instead of
     through torch.distributed.  Returns the number of exchange rounds."""
-    for s in strips:
-        s.start(goal_global)
+    pending = [s.start(goal_global, phases_per_round) for s in strips]
     rounds = 0
     while rounds < max_rounds:
         rows = [tuple(r.clone() for r in s.boundary_rows()) for s in strips]
@@ -247,26 +206,6 @@ def dd_solve_lockstep(strips, goal_global, max_rounds=10000):
             from_above = rows[k - 1][1] if k > 0 else None
             from_below = rows[k + 1][0] if k + 1 < len(strips) else None
             todo.append(s.absorb(from_above, from_below))
-        if not any(todo):
-            break
-        for s, ranges in zip(strips, todo):
-            if ranges:
-                s.resume(ranges)
-    return rounds
-
-
-def dd_solve_lockstep_pipelined(strips, goal_global, phases_per_round=16, max_rounds=1000000):
-    """dd_solve_pipelined with all strips in one process (see dd_solve_lockstep)."""
-    pending = [s.start_bounded(goal_global, phases_per_round) for s in strips]
-    rounds = 0
-    while rounds < max_rounds:
-        rows = [tuple(r.clone() for r in s.boundary_rows()) for s in strips]
-        rounds += 1
-        todo = []
-        for k, s in enumerate(strips):
-            from_above = rows[k - 1][1] if k > 0 else None
-            from_below = rows[k + 1][0] if k + 1 < len(strips) else None
-            todo.append(s.absorb_keyed(from_above, from_below))
         if not any(pending) and not any(r for r, _ in todo):
             break
         pending = [s.advance(r, key, phases_per_round) for s, (r, key) in zip(strips, todo)]

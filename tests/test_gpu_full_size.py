@@ -68,7 +68,7 @@ def test_plan4096_is_the_exact_fixed_point(pkg):
     assert np.count_nonzero(gap) <= 0.02 * gap.size
     del Tn
     # idempotence: waking every tile again leaves the plane bit-identical
-    again = dev.solve_resume([(0, n)])
+    again = dev.solve_advance([(0, n)], 0.0, 1 << 20)
     assert again["converged"] and again["tile_activations"] >= (n // 32) ** 2
     assert np.array_equal(dev.download_total_cost(), T)
     # the path descends strictly and arrives

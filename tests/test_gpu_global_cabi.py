@@ -181,7 +181,7 @@ def test_abandoned_bounded_solve_leaves_no_stale_wakeups(pkg):
     assert np.array_equal(np.isinf(got), np.isinf(want))
     fin = np.isfinite(want) & (want > 0)
     assert np.max(np.abs(got[fin] - want[fin]) / want[fin]) <= 1e-13
-    # the same after reset_total_cost() and after a resume that drops the pending work
+    # the same after reset_total_cost() dropped the pending work of a phase-bounded solve
     st = dut.solve_start(ga, 2)
     dut.reset_total_cost()
     assert dut.solve_total_cost([gb])["converged"]

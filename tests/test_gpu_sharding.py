@@ -7,31 +7,12 @@ from conftest import rel_err
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.mark.parametrize("k", [2, 3, 4])
-def test_k_strips_equal_single_grid(pkg, k):
-    import torch
-    sh, api, syn = pkg.sharding, pkg.cuda_api, pkg.synthetic
-    ny, nx = 384, 320
-    cost = syn.smooth_cost_map(ny, nx, seed=21, obstacle_fraction=0.04)
-    gi, gj = syn.free_interior_cell_near(cost <= 0, 200, 40)
-    whole = api.DeviceLayer(nx, ny)
-    whole.set_cost_map(cost)
-    whole.solve_total_cost([(gi, gj)])
-    T1 = whole.download_total_cost()
-    strips = []
-    for r in range(k):
-        lay = sh.StripLayout(ny, k, r)
-        strips.append(sh.CudaStrip(api, lay, nx, cost[lay.r0:lay.r1], 0, torch))
-    rounds = sh.dd_solve_lockstep(strips, (gi, gj))
-    Tk = np.vstack([s.own_rows() for s in strips])
-    assert rounds >= 2
-    assert np.array_equal(np.isinf(Tk), np.isinf(T1))
-    assert rel_err(Tk, T1) <= 1e-12
+UNBOUNDED = 10**6   # a phase budget no strip exhausts: every strip converges before it trades rows
 
 
-def test_batched_slots_resume_and_rows(pkg):
-    """export/import round trip and resume after lowering a row by hand."""
+def test_batched_slots_advance_and_rows(pkg):
+    """export/import round trip, then a solve_advance on the clean work list of a converged solve
+    wakes the tiles of a row lowered by hand."""
     import torch
     api = pkg.cuda_api
     n = 128
@@ -43,9 +24,9 @@ def test_batched_slots_resume_and_rows(pkg):
     dev.export_rows(10, 1, row.data_ptr(), True)
     assert np.array_equal(row.cpu().numpy(), T0[10])
     lower = torch.full((n,), 0.5, dtype=torch.float64, device="cuda")
-    assert dev.import_rows_min(10, 1, lower.data_ptr(), True)
-    assert not dev.import_rows_min(10, 1, lower.data_ptr(), True)
-    dev.solve_resume([(9, 12)])
+    assert dev.import_rows_min_key(10, 1, lower.data_ptr(), True) == (True, 0.5)
+    assert dev.import_rows_min_key(10, 1, lower.data_ptr(), True) == (False, float("inf"))
+    assert dev.solve_advance([(9, 12)], 0.5, 1 << 20)["converged"]
     T1 = dev.download_total_cost()
     assert np.all(T1 <= T0) and T1[11, 5] == 1.5 and T1[10, 5] == 0.5
 
@@ -83,13 +64,16 @@ def test_phase_bounded_solve_equals_one_shot(pkg, phases):
     assert again["converged"] and again["tile_activations"] == 0
 
 
-@pytest.mark.parametrize("k,phases", [(2, 3), (3, 8), (4, 2)])
-def test_pipelined_strips_equal_single_grid(pkg, k, phases):
+# goal row 180: the goal lies in an interior strip for k >= 3; goal row 40: in the first strip, so
+# with an unbounded budget the converged front of one strip after the other crosses every cut
+@pytest.mark.parametrize("k,phases,goal_row", [(2, 3, 180), (3, 8, 180), (4, 2, 180),
+                                               (2, UNBOUNDED, 40), (3, UNBOUNDED, 40), (4, UNBOUNDED, 40)])
+def test_pipelined_strips_equal_single_grid(pkg, k, phases, goal_row):
     import torch
     sh, api, syn = pkg.sharding, pkg.cuda_api, pkg.synthetic
     ny, nx = 384, 320
     cost = syn.smooth_cost_map(ny, nx, seed=21, obstacle_fraction=0.04)
-    gi, gj = syn.free_interior_cell_near(cost <= 0, 200, 180)   # goal in an interior strip for k >= 3
+    gi, gj = syn.free_interior_cell_near(cost <= 0, 200, goal_row)
     whole = api.DeviceLayer(nx, ny)
     whole.set_cost_map(cost)
     whole.solve_total_cost([(gi, gj)])
@@ -98,7 +82,7 @@ def test_pipelined_strips_equal_single_grid(pkg, k, phases):
     for r in range(k):
         lay = sh.StripLayout(ny, k, r)
         strips.append(sh.CudaStrip(api, lay, nx, cost[lay.r0:lay.r1], 0, torch))
-    rounds = sh.dd_solve_lockstep_pipelined(strips, (gi, gj), phases_per_round=phases)
+    rounds = sh.dd_solve_lockstep(strips, (gi, gj), phases_per_round=phases)
     Tk = np.vstack([s.own_rows() for s in strips])
     assert rounds >= 2
     assert np.array_equal(np.isinf(Tk), np.isinf(T1))
