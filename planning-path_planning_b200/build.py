@@ -75,6 +75,8 @@ def build_cuda(force=False, verbose=False, ptxas_v=False):
                 extra.append("-DDYMU_FIM_PROFILE")
             if os.environ.get("DYMU_LOCAL_PROFILE"):
                 extra.append("-DDYMU_LOCAL_PROFILE")
+            if os.environ.get("DYMU_PATH_PROFILE"):
+                extra.append("-DDYMU_PATH_PROFILE")
             log += _run([NVCC] + NVCC_FLAGS + extra + ["-c", src, "-o", obj], verbose)
     if force or _newer(CUDA_SO, objs):
         _run([NVCC, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-ccbin", CXX,
