@@ -50,6 +50,12 @@ typedef struct dymu_ctx dymu_ctx;
 #define DYMU_PLANE_TRAFFICABILITY 5
 #define DYMU_PLANE_TOTAL_COST 6 /* slot 0; other slots through dymu_download_total_cost */
 #define DYMU_PLANE_CEFF 7       /* global_res*cost*(2+hazard-trafficability), obstacle = +inf */
+/* directional costs a(x->m) of the anisotropic solve, toward the neighbour at i-1, i+1, j-1,
+ * j+1 (see dymu_set_anisotropy).  Read-only; they exist only while anisotropy is on. */
+#define DYMU_PLANE_DIRCOST_XM 8
+#define DYMU_PLANE_DIRCOST_XP 9
+#define DYMU_PLANE_DIRCOST_YM 10
+#define DYMU_PLANE_DIRCOST_YP 11
 /* byte / word planes */
 #define DYMU_PLANE_U8_OBSTACLE 0
 #define DYMU_PLANE_U8_LOCMODE 1 /* index into locomotion_modes, 255 = "DONT_CARE" */
@@ -138,6 +144,26 @@ int dymu_compute_cost_map(dymu_ctx* ctx, const double* cost_lut, int n_lut, cons
                           int n_slopes, int n_locs, const double* elevation, size_t ld_e,
                           const double* terrain, size_t ld_t);
 int dymu_upload_terrain(dymu_ctx* ctx, const double* terrain, size_t ld);
+
+/* ---- slope anisotropy (an extension; the reference's update is isotropic) -------------
+ * n >= 2 pairs (theta_deg[k], factor[k]): signed slope angle in degrees, strictly ascending,
+ * positive = uphill in the direction of travel; factor finite and > 0.  f(theta) is piecewise
+ * linear in the table and clamped at both ends:
+ *     f = factor[k] + (factor[k+1]-factor[k]) * ((theta-theta_deg[k]) / (theta_deg[k+1]-theta_deg[k]))
+ * for theta_deg[k] <= theta < theta_deg[k+1].  For a cell x and its 4-neighbour m
+ *     theta(x->m) = atan((elev[m]-elev[x]) / global_res) * (180/pi)
+ *     a(x->m)     = C_eff(x) * f(theta(x->m))      (C_eff: DYMU_PLANE_CEFF; +inf toward outside)
+ * and the total-cost update of x is the smallest of the four one-sided values T[m] + a(x->m)
+ * and, for each pair (h in {i-1,i+1}, v in {j-1,j+1}) with -a_h < T_h - T_v < a_v, the root
+ *     ((a_v^2*T_h + a_h^2*T_v) + (a_h*a_v)*sqrt((a_h^2+a_v^2) - d^2)) / (a_h^2+a_v^2),  d = T_h-T_v.
+ * The descent scales the per-axis differences of gradientNode by 1/a^2 of the move against
+ * them and normalises (DESIGN.md section 10).  While on, dymu_solve_total_cost,
+ * dymu_solve_incremental (always a full solve), dymu_plan_streamed (upload first, then the full
+ * solve), the path extraction and dymu_batch_solve are anisotropic; dymu_solve_start,
+ * dymu_solve_advance and dymu_dd_solve return DYMU_ERR_STATE.  n = 0 switches it off and frees
+ * the directional-cost planes; any other malformed table is DYMU_ERR_ARG. */
+#define DYMU_ANISO_MAX 64
+int dymu_set_anisotropy(dymu_ctx* ctx, const double* theta_deg, const double* factor, int n);
 
 /* ---- total-cost solve -------------------------------------------------------- */
 /* Number of independent total-cost planes ("slots") for batched goal queries. */

@@ -151,6 +151,10 @@ int dymu_planner_propagate_global_node(dymu_planner* p, unsigned i, unsigned j, 
 int dymu_planner_set_cost_map_flat(dymu_planner* p, const double* cost, unsigned ld);
 int dymu_planner_set_total_cost_target(dymu_planner* p, double* out, unsigned ld);
 int dymu_planner_get_total_cost_matrix_flat(dymu_planner* p, double* out, unsigned ld);
+/* setSlopeAnisotropy(angles, factors) (extension of the B200 drop-in): n pairs of signed slope
+ * angle in degrees and cost factor, n = 0 switches it off; 1 = applied, 0 = rejected.  The
+ * reference has no such capability: its build returns -1. */
+int dymu_planner_set_slope_anisotropy(dymu_planner* p, const double* angles, const double* factors, int n);
 
 double dymu_planner_last_call_seconds(dymu_planner* p);
 

@@ -439,6 +439,18 @@ int dymu_planner_propagate_global_node(dymu_planner* p, unsigned i, unsigned j, 
     return 1;
 }
 
+int dymu_planner_set_slope_anisotropy(dymu_planner* p, const double* angles, const double* factors, int n)
+{
+    if (!p || n < 0 || (n > 0 && (!angles || !factors))) return -1;
+#if defined(DYMU_CAPI_B200)
+    std::vector<double> a(angles, angles + n), f(factors, factors + n);
+    Stopwatch sw(&p->last_seconds);
+    return p->impl->setSlopeAnisotropy(a, f) ? 1 : 0;
+#else
+    return -1;  // the reference's update is isotropic
+#endif
+}
+
 int dymu_planner_set_cost_map_flat(dymu_planner* p, const double* cost, unsigned ld)
 {
     if (!p || !cost || ld < p->nx) return -1;

@@ -171,7 +171,9 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
     if (!ctx || goal_i >= ctx->nx || goal_j >= ctx->ny) return DYMU_ERR_ARG;
     if (cells_invalidated) *cells_invalidated = UINT64_MAX;  // "everything": a full solve ran
     const size_t n = (size_t)ctx->pitch * ctx->rows;
-    const bool reusable = ctx->solved && ctx->last_n_goals == 1 && ctx->last_goal_i == goal_i
+    // the anisotropic solve has no invalidation cone: a change of C_eff or of the elevation moves
+    // the directional costs of the cell and of its neighbours' pairs
+    const bool reusable = !ctx->aniso_n && ctx->solved && ctx->last_n_goals == 1 && ctx->last_goal_i == goal_i
                           && ctx->last_goal_j == goal_j && !ctx->work.unclean && ctx->have_cost
                           && n < ((size_t)1 << 32);
     if (!reusable) return dymu_solve_total_cost(ctx, 1, &goal_i, &goal_j, stats);

@@ -17,7 +17,11 @@
 // it has the helpers build a window around its cell and waits.  Every lane of the walker
 // carries the identical waypoint state (no divergence); lane 0 stores the waypoint.  Batches
 // of queries run one CTA per query.
+// With slope anisotropy on (dymu_set_anisotropy) the helpers put the characteristic direction
+// of the anisotropic metric into the window instead of the normalised gradient; the walker is
+// the same.
 #include <limits.h>
+#include <type_traits>
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -49,6 +53,13 @@ struct PathArgs
 #ifdef DYMU_PATH_PROFILE
     unsigned long long* prof;  // walk cycles, window cycles, windows, missed prefetches (single calls)
 #endif
+};
+
+// the anisotropic descent also reads the directional-cost planes (order i-1, i+1, j-1, j+1)
+struct PathArgsAniso : PathArgs
+{
+    const double* A;
+    size_t a_stride;  // doubles between two of those planes
 };
 
 // per-axis rule of gradientNode (G.cpp:722-761); lo/hi missing = NULL neighbour
@@ -87,7 +98,13 @@ __device__ __forceinline__ void bar_sync(int id)
 // helper warps: elevation and the normalised gradient of gradientNode (G.cpp:718-772) of
 // every node of the window at (x0, y0) whose stencil is inside it; the total cost is read from
 // L2.  A thread puts the loads of BUILD_BATCH nodes in flight before it computes any of them.
-__device__ __forceinline__ void build_window(const PathArgs& a, double* wb, int x0, int y0,
+// ANISO: each difference is scaled by 1/a^2 of the move against it -- a(x->i-1) when it is
+// positive, a(x->i+1) otherwise, likewise for y -- before the normalisation; a component that is
+// 0 or whose cost is +inf (a neighbour outside the grid) is 0.  (p_x/a_x^2, p_y/a_y^2) is the
+// characteristic direction of the metric; with f = 1 it is the normalised gradient up to
+// rounding.  An impassable node (all four costs +inf) has no metric and keeps the gradient.
+template <bool ANISO, class Args>
+__device__ __forceinline__ void build_window(const Args& a, double* wb, int x0, int y0,
                                              const volatile int* stop)
 {
     const int t = threadIdx.x - 32;
@@ -96,6 +113,7 @@ __device__ __forceinline__ void build_window(const PathArgs& a, double* wb, int 
         if (*stop) return;
         double f[BUILD_BATCH], fl[BUILD_BATCH], fr[BUILD_BATCH], fd[BUILD_BATCH], fu[BUILD_BATCH];
         double ev[BUILD_BATCH];
+        double axm[BUILD_BATCH], axp[BUILD_BATCH], aym[BUILD_BATCH], ayp[BUILD_BATCH];
         bool hl[BUILD_BATCH], hr[BUILD_BATCH], hd[BUILD_BATCH], hu[BUILD_BATCH], inner[BUILD_BATCH];
 #pragma unroll
         for (int u = 0; u < BUILD_BATCH; ++u)
@@ -120,6 +138,13 @@ __device__ __forceinline__ void build_window(const PathArgs& a, double* wb, int 
                 if (hr[u]) fr[u] = __ldcg(Tc + 1);
                 if (hd[u]) fd[u] = __ldcg(Tc - a.pitch);
                 if (hu[u]) fu[u] = __ldcg(Tc + a.pitch);
+                if constexpr (ANISO)
+                {
+                    axm[u] = __ldg(a.A + at);
+                    axp[u] = __ldg(a.A + a.a_stride + at);
+                    aym[u] = __ldg(a.A + 2 * a.a_stride + at);
+                    ayp[u] = __ldg(a.A + 3 * a.a_stride + at);
+                }
             }
         }
 #pragma unroll
@@ -129,8 +154,18 @@ __device__ __forceinline__ void build_window(const PathArgs& a, double* wb, int 
             double dnx = 0, dny = 0;
             if (inner[u])
             {
-                const double dx = grad_axis(f[u], hl[u], fl[u], hr[u], fr[u]);
-                const double dy = grad_axis(f[u], hd[u], fd[u], hu[u], fu[u]);
+                double dx = grad_axis(f[u], hl[u], fl[u], hr[u], fr[u]);
+                double dy = grad_axis(f[u], hd[u], fd[u], hu[u], fu[u]);
+                if constexpr (ANISO)
+                {
+                    const double inf = DYMU_INF;
+                    if (!(axm[u] == inf && axp[u] == inf && aym[u] == inf && ayp[u] == inf))
+                    {
+                        const double ax = dx > 0 ? axm[u] : axp[u], ay = dy > 0 ? aym[u] : ayp[u];
+                        dx = (dx == 0 || ax == inf) ? 0.0 : dx / (ax * ax);
+                        dy = (dy == 0 || ay == inf) ? 0.0 : dy / (ay * ay);
+                    }
+                }
                 if (!((dx == 0) && (dy == 0)))
                 {
                     const double nrm = sqrt(dx * dx + dy * dy);
@@ -252,10 +287,10 @@ __device__ double sqrt_lt_threshold(double c)
 }
 
 // computeGlobalPath, G.cpp:615-662
-template <bool UNIT_RES>
-__global__ void __launch_bounds__(PATH_THREADS, 1) k_global_path(const PathArgs* args_arr)
+template <bool UNIT_RES, bool ANISO = false, class Args = std::conditional_t<ANISO, PathArgsAniso, PathArgs>>
+__global__ void __launch_bounds__(PATH_THREADS, 1) k_global_path(const Args* args_arr)
 {
-    const PathArgs a = args_arr[blockIdx.x];
+    const Args a = args_arr[blockIdx.x];
     extern __shared__ __align__(16) double path_smem[];  // two windows of WIN_DOUBLES
     __shared__ WinCmd cmd;
     if (threadIdx.x >= 32)
@@ -266,7 +301,7 @@ __global__ void __launch_bounds__(PATH_THREADS, 1) k_global_path(const PathArgs*
             bar_sync(BAR_CMD);
             const int x0 = cmd.x0, y0 = cmd.y0, buf = cmd.buf;
             if (x0 == INT_MIN) return;
-            build_window(a, path_smem + buf * WIN_DOUBLES, x0, y0, &cmd.stop);
+            build_window<ANISO>(a, path_smem + buf * WIN_DOUBLES, x0, y0, &cmd.stop);
             bar_arrive(BAR_DONE);
         }
     }
@@ -408,12 +443,37 @@ __global__ void __launch_bounds__(PATH_THREADS, 1) k_global_path(const PathArgs*
     }
 }
 
-int launch_paths(dymu_ctx* ctx, uint32_t n, const PathArgs* d_args)
+template <class Args> int launch_paths_as(dymu_ctx* ctx, uint32_t n, const Args* d_args)
 {
-    auto kernel = (ctx->gres == 1.0) ? k_global_path<true> : k_global_path<false>;
+    constexpr bool aniso = std::is_same<Args, PathArgsAniso>::value;
+    auto kernel = (ctx->gres == 1.0) ? k_global_path<true, aniso> : k_global_path<false, aniso>;
     DYMU_CUDA_TRY(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PATH_SMEM));
     kernel<<<n, PATH_THREADS, PATH_SMEM, ctx->stream>>>(d_args);
     return DYMU_OK;
+}
+
+// d_args: n argument blocks of args_size(ctx) bytes each
+int launch_paths(dymu_ctx* ctx, uint32_t n, const void* d_args)
+{
+    if (ctx->aniso_n) return launch_paths_as(ctx, n, (const PathArgsAniso*)d_args);
+    return launch_paths_as(ctx, n, (const PathArgs*)d_args);
+}
+
+size_t args_size(const dymu_ctx* ctx) { return ctx->aniso_n ? sizeof(PathArgsAniso) : sizeof(PathArgs); }
+
+// the argument block of one query in the form the kernel of the context's mode takes
+void put_args(const dymu_ctx* ctx, const PathArgs& a, void* dst)
+{
+    if (ctx->aniso_n)
+    {
+        PathArgsAniso x;
+        static_cast<PathArgs&>(x) = a;
+        x.A = ctx->dircost;
+        x.a_stride = (size_t)ctx->pitch * ctx->rows;
+        memcpy(dst, &x, sizeof(x));
+    }
+    else
+        memcpy(dst, &a, sizeof(a));
 }
 }  // namespace
 
@@ -428,8 +488,9 @@ int dymu_extract_global_path(dymu_ctx* ctx, uint32_t slot, double x0, double y0,
     if (goal_i >= ctx->nx || goal_j >= ctx->ny) return DYMU_ERR_ARG;
     size_t out_bytes = (size_t)cap * 5 * sizeof(double);
     size_t hdr = 256;
+    if (ctx->aniso_n) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
     DYMU_TRY(dymu_internal_scratch(ctx, hdr + out_bytes, hdr + out_bytes));
-    PathArgs* h_args = (PathArgs*)ctx->h_pinned;
+    const size_t asz = args_size(ctx);
     PathArgs a;
     a.T = ctx->T + (size_t)slot * ctx->pitch * ctx->rows;
     a.elev = ctx->elev;
@@ -438,20 +499,19 @@ int dymu_extract_global_path(dymu_ctx* ctx, uint32_t slot, double x0, double y0,
     a.goal_i = goal_i; a.goal_j = goal_j;
     a.out = (double*)((char*)ctx->d_scratch + hdr);
     a.cap = cap;
-    a.result = (uint32_t*)((char*)ctx->d_scratch + sizeof(PathArgs));
+    a.result = (uint32_t*)((char*)ctx->d_scratch + asz);
 #ifdef DYMU_PATH_PROFILE
-    a.prof = (unsigned long long*)((char*)ctx->d_scratch + sizeof(PathArgs) + 8);
-    static_assert(sizeof(PathArgs) + 8 + 4 * 8 <= 256, "path header overflow");
+    a.prof = (unsigned long long*)((char*)ctx->d_scratch + asz + 8);
+    static_assert(sizeof(PathArgsAniso) + 8 + 4 * 8 <= 256, "path header overflow");
 #else
-    static_assert(sizeof(PathArgs) + 8 <= 256, "path header overflow");
+    static_assert(sizeof(PathArgsAniso) + 8 <= 256, "path header overflow");
 #endif
-    *h_args = a;
-    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_scratch, h_args, sizeof(PathArgs),
-                                       cudaMemcpyHostToDevice, ctx->stream));
-    DYMU_TRY(launch_paths(ctx, 1, (const PathArgs*)ctx->d_scratch));
+    put_args(ctx, a, ctx->h_pinned);
+    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_scratch, ctx->h_pinned, asz, cudaMemcpyHostToDevice, ctx->stream));
+    DYMU_TRY(launch_paths(ctx, 1, ctx->d_scratch));
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
-    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + sizeof(PathArgs));
+    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + asz);
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h_res, a.result, 8, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     *n_out = h_res[0];
@@ -459,7 +519,7 @@ int dymu_extract_global_path(dymu_ctx* ctx, uint32_t slot, double x0, double y0,
 #ifdef DYMU_PATH_PROFILE
     if (getenv("DYMU_TRACE_CALLS"))
     {
-        unsigned long long* h_prof = (unsigned long long*)((char*)ctx->h_pinned + sizeof(PathArgs) + 8);
+        unsigned long long* h_prof = (unsigned long long*)((char*)ctx->h_pinned + asz + 8);
         DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h_prof, a.prof, 4 * 8, cudaMemcpyDeviceToHost, ctx->stream));
         DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
         fprintf(stderr, "[dymu]   path: %u waypoints, walk %llu cycles, windows %llu cycles for %llu windows "
@@ -485,12 +545,14 @@ int dymu_extract_global_path_batch(dymu_ctx* ctx, uint32_t n, const uint32_t* sl
     for (uint32_t q = 0; q < n; ++q)
         if (slots[q] >= ctx->n_slots || goal_ij[2 * q] >= ctx->nx || goal_ij[2 * q + 1] >= ctx->ny)
             return DYMU_ERR_ARG;
-    const size_t hdr = (((size_t)n * (sizeof(PathArgs) + 8)) + 255) & ~(size_t)255;
+    if (ctx->aniso_n) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
+    const size_t asz = args_size(ctx);
+    const size_t hdr = (((size_t)n * (asz + 8)) + 255) & ~(size_t)255;
     const size_t out_bytes = (size_t)n * cap * 5 * sizeof(double);
     DYMU_TRY(dymu_internal_scratch(ctx, hdr + out_bytes, hdr));
-    PathArgs* h_args = (PathArgs*)ctx->h_pinned;
+    char* h_args = (char*)ctx->h_pinned;
     char* d_base = (char*)ctx->d_scratch;
-    uint32_t* d_res = (uint32_t*)(d_base + (size_t)n * sizeof(PathArgs));
+    uint32_t* d_res = (uint32_t*)(d_base + (size_t)n * asz);
     for (uint32_t q = 0; q < n; ++q)
     {
         PathArgs a;
@@ -505,14 +567,13 @@ int dymu_extract_global_path_batch(dymu_ctx* ctx, uint32_t n, const uint32_t* sl
 #ifdef DYMU_PATH_PROFILE
         a.prof = nullptr;
 #endif
-        h_args[q] = a;
+        put_args(ctx, a, h_args + (size_t)q * asz);
     }
-    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(d_base, h_args, (size_t)n * sizeof(PathArgs), cudaMemcpyHostToDevice,
-                                       ctx->stream));
-    DYMU_TRY(launch_paths(ctx, n, (const PathArgs*)d_base));
+    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(d_base, h_args, (size_t)n * asz, cudaMemcpyHostToDevice, ctx->stream));
+    DYMU_TRY(launch_paths(ctx, n, d_base));
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
-    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + (size_t)n * sizeof(PathArgs));
+    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + (size_t)n * asz);
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h_res, d_res, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (uint32_t q = 0; q < n; ++q)

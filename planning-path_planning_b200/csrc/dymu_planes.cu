@@ -263,6 +263,74 @@ __global__ void k_ceff_stats(const double* __restrict__ ceff, size_t n, double* 
     }
 }
 
+// the factor table of the anisotropic solve, passed by value (it lives in the constant bank)
+struct AnisoTable
+{
+    int n;
+    double theta[DYMU_ANISO_MAX], f[DYMU_ANISO_MAX];
+};
+
+// f(theta): piecewise linear in the table, clamped at both ends (restated by
+// the test oracle in the same expression order)
+__device__ __forceinline__ double aniso_factor(const AnisoTable& t, double th)
+{
+    if (th <= t.theta[0]) return t.f[0];
+    if (th >= t.theta[t.n - 1]) return t.f[t.n - 1];
+    int k = 0;
+    while (th >= t.theta[k + 1]) ++k;
+    return t.f[k] + (t.f[k + 1] - t.f[k]) * ((th - t.theta[k]) / (t.theta[k + 1] - t.theta[k]));
+}
+
+// Directional costs of the anisotropic solve, all four planes of every padded cell:
+//     a(x->m) = C_eff(x) * f(atan((elev[m] - elev[x]) / gres) * (180/pi))
+// toward m = i-1, i+1, j-1, j+1; +inf where C_eff(x) is +inf (obstacles, padding) and toward a
+// neighbour outside the grid.  16 B read + 32 B written per cell (the neighbours' elevations come
+// from cache).  Accumulates sum and count of the finite values: the band width of the solver.
+__global__ void k_dircost(const double* __restrict__ elev, const double* __restrict__ ceff,
+                          double* __restrict__ A, size_t plane, double gres, uint32_t pitch, uint32_t rows,
+                          uint32_t nx, uint32_t ny, AnisoTable tab, double* stats)
+{
+    constexpr double kDeg = 180.0 / 3.141592653589793;
+    const size_t total = (size_t)pitch * rows;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    double sum = 0, cnt = 0;
+    for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < total; q += stride)
+    {
+        const uint32_t j = (uint32_t)(q / pitch), i = (uint32_t)(q % pitch);
+        const double c = ceff[q];
+        double a[4] = {DYMU_INF, DYMU_INF, DYMU_INF, DYMU_INF};
+        if (c < DYMU_INF && i < nx && j < ny)
+        {
+            const double e = elev[q];
+            const bool has[4] = {i > 0, i + 1 < nx, j > 0, j + 1 < ny};
+            const ptrdiff_t off[4] = {-1, 1, -(ptrdiff_t)pitch, (ptrdiff_t)pitch};
+#pragma unroll
+            for (int d = 0; d < 4; ++d)
+                if (has[d])
+                {
+                    a[d] = c * aniso_factor(tab, atan((elev[q + off[d]] - e) / gres) * kDeg);
+                    if (a[d] < DYMU_INF)
+                    {
+                        sum += a[d];
+                        cnt += 1.0;
+                    }
+                }
+        }
+#pragma unroll
+        for (int d = 0; d < 4; ++d) A[d * plane + q] = a[d];
+    }
+    for (int o = 16; o > 0; o >>= 1)
+    {
+        sum += __shfl_down_sync(0xffffffffu, sum, o);
+        cnt += __shfl_down_sync(0xffffffffu, cnt, o);
+    }
+    if ((threadIdx.x & 31) == 0 && cnt > 0)
+    {
+        atomicAdd(&stats[0], sum);
+        atomicAdd(&stats[1], cnt);
+    }
+}
+
 // dense read-back with the getter transforms of G.cpp:799-829.  8(+17) B read, 8 B written.
 __global__ void k_readback(const double* __restrict__ src, const double* __restrict__ haz,
                            const double* __restrict__ traff, const uint8_t* __restrict__ obst,
@@ -340,6 +408,13 @@ double* plane_ptr(dymu_ctx* ctx, int plane)
         case DYMU_PLANE_TRAFFICABILITY: return ctx->traff;
         case DYMU_PLANE_TOTAL_COST: return ctx->T;
         case DYMU_PLANE_CEFF: return ctx->ceff;
+        case DYMU_PLANE_DIRCOST_XM:
+        case DYMU_PLANE_DIRCOST_XP:
+        case DYMU_PLANE_DIRCOST_YM:
+        case DYMU_PLANE_DIRCOST_YP:
+            // only while anisotropy is on
+            return ctx->dircost ? ctx->dircost + (size_t)(plane - DYMU_PLANE_DIRCOST_XM) * ctx->pitch * ctx->rows
+                                : nullptr;
         default: return nullptr;
     }
 }
@@ -359,6 +434,15 @@ int fill_plane(dymu_ctx* ctx, double* p, double v, size_t n)
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
     return DYMU_OK;
+}
+
+bool is_dircost(int plane) { return plane >= DYMU_PLANE_DIRCOST_XM && plane <= DYMU_PLANE_DIRCOST_YP; }
+
+// planes C_eff (and, while anisotropy is on, the directional costs) are built from
+bool feeds_ceff(const dymu_ctx* ctx, int plane)
+{
+    return plane == DYMU_PLANE_COST || plane == DYMU_PLANE_HAZARD_DENSITY || plane == DYMU_PLANE_TRAFFICABILITY
+           || (ctx->aniso_n && plane == DYMU_PLANE_ELEVATION);
 }
 }  // namespace
 
@@ -384,6 +468,8 @@ int dymu_internal_scratch(dymu_ctx* ctx, size_t dev_bytes, size_t host_bytes)
     }
     return DYMU_OK;
 }
+
+static int build_dircost(dymu_ctx* ctx);
 
 extern "C" {
 
@@ -471,7 +557,7 @@ int dymu_destroy(dymu_ctx* ctx)
     dymu_internal_fim_free(&ctx->work);
     void* ptrs[] = {ctx->elev, ctx->slope, ctx->raw, ctx->cost, ctx->haz, ctx->traff, ctx->ceff,
                     ctx->T, ctx->terrain, ctx->obst, ctx->locmode, ctx->d_lut, ctx->d_slopes,
-                    ctx->d_stage, ctx->d_scratch, ctx->tile_tmax, ctx->d_upflag};
+                    ctx->d_stage, ctx->d_scratch, ctx->tile_tmax, ctx->d_upflag, ctx->dircost};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
@@ -538,6 +624,7 @@ int dymu_upload_plane(dymu_ctx* ctx, int plane, const double* host, size_t ld)
 {
     DYMU_GUARD(ctx);
     if (!ctx || !host || ld < ctx->nx) return DYMU_ERR_ARG;
+    if (is_dircost(plane)) DYMU_FAIL(ctx, DYMU_ERR_ARG, "the directional-cost planes are read-only");
     double* d = plane_ptr(ctx, plane);
     if (!d) DYMU_FAIL(ctx, DYMU_ERR_ARG, "unknown plane %d", plane);
     if (plane == DYMU_PLANE_TOTAL_COST) DYMU_TRY(dymu_internal_settle_delivery(ctx));
@@ -545,9 +632,7 @@ int dymu_upload_plane(dymu_ctx* ctx, int plane, const double* host, size_t ld)
                                          ctx->nx * sizeof(double), ctx->ny, cudaMemcpyHostToDevice,
                                          ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (plane == DYMU_PLANE_COST || plane == DYMU_PLANE_HAZARD_DENSITY
-        || plane == DYMU_PLANE_TRAFFICABILITY)
-        ctx->ceff_dirty = true;
+    if (feeds_ceff(ctx, plane)) ctx->ceff_dirty = true;
     if (plane == DYMU_PLANE_TOTAL_COST) ctx->solved = ctx->export_done = false;
     return DYMU_OK;
 }
@@ -602,7 +687,7 @@ int dymu_download_plane(dymu_ctx* ctx, int plane, double* host, size_t ld, int x
 {
     DYMU_GUARD(ctx);
     if (!ctx || !host || ld < ctx->nx) return DYMU_ERR_ARG;
-    if (plane == DYMU_PLANE_CEFF) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
+    if (plane == DYMU_PLANE_CEFF || is_dircost(plane)) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
     double* d = plane_ptr(ctx, plane);
     if (!d) DYMU_FAIL(ctx, DYMU_ERR_ARG, "unknown plane %d", plane);
     return download_f64(ctx, d, host, ld, xform);
@@ -703,7 +788,7 @@ int dymu_read_rect(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32_t 
 {
     DYMU_GUARD(ctx);
     if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h)) return DYMU_ERR_ARG;
-    if (plane == DYMU_PLANE_CEFF) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
+    if (plane == DYMU_PLANE_CEFF || is_dircost(plane)) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     DYMU_CUDA_TRY(ctx, cudaMemcpy2DAsync(host, w * sizeof(double), d + (size_t)j0 * ctx->pitch + i0,
@@ -717,7 +802,7 @@ int dymu_write_rect(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32_t
                     const double* host)
 {
     DYMU_GUARD(ctx);
-    if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h)) return DYMU_ERR_ARG;
+    if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h) || is_dircost(plane)) return DYMU_ERR_ARG;
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     if (plane == DYMU_PLANE_TOTAL_COST) DYMU_TRY(dymu_internal_settle_delivery(ctx));
@@ -726,9 +811,7 @@ int dymu_write_rect(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32_t
                                          w * sizeof(double), h, cudaMemcpyHostToDevice,
                                          ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (plane == DYMU_PLANE_COST || plane == DYMU_PLANE_HAZARD_DENSITY
-        || plane == DYMU_PLANE_TRAFFICABILITY)
-        ctx->ceff_dirty = true;
+    if (feeds_ceff(ctx, plane)) ctx->ceff_dirty = true;
     if (plane == DYMU_PLANE_TOTAL_COST) ctx->solved = ctx->export_done = false;  // no longer the solver's fixed point
     return DYMU_OK;
 }
@@ -749,14 +832,12 @@ int dymu_read_rect_u8(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32
 int dymu_plane_device_ptr(dymu_ctx* ctx, int plane, void** dptr, size_t* pitch_elems)
 {
     DYMU_GUARD(ctx);
-    if (!ctx || !dptr) return DYMU_ERR_ARG;
+    if (!ctx || !dptr || is_dircost(plane)) return DYMU_ERR_ARG;
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     *dptr = d;
     if (pitch_elems) *pitch_elems = ctx->pitch;
-    if (plane == DYMU_PLANE_COST || plane == DYMU_PLANE_HAZARD_DENSITY
-        || plane == DYMU_PLANE_TRAFFICABILITY)
-        ctx->ceff_dirty = true;  // the caller may write through the pointer
+    if (feeds_ceff(ctx, plane)) ctx->ceff_dirty = true;  // the caller may write through the pointer
     return DYMU_OK;
 }
 
@@ -932,6 +1013,45 @@ int dymu_read_node(dymu_ctx* ctx, uint32_t i, uint32_t j, double out[10])
     return DYMU_OK;
 }
 
+int dymu_set_anisotropy(dymu_ctx* ctx, const double* theta_deg, const double* factor, int n)
+{
+    DYMU_GUARD(ctx);
+    if (!ctx || n < 0) return DYMU_ERR_ARG;
+    if (n == 0)
+    {
+        if (ctx->aniso_n)
+        {
+            DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            cudaFree(ctx->dircost);
+            ctx->dircost = nullptr;
+            ctx->aniso_n = 0;
+            ctx->solved = false;  // the resident map is not the isotropic fixed point
+        }
+        return DYMU_OK;
+    }
+    if (n < 2 || n > DYMU_ANISO_MAX || !theta_deg || !factor)
+        DYMU_FAIL(ctx, DYMU_ERR_ARG, "anisotropy table: need 2..%d pairs", DYMU_ANISO_MAX);
+    for (int k = 0; k < n; ++k)
+    {
+        if (!isfinite(theta_deg[k]) || !isfinite(factor[k]) || !(factor[k] > 0))
+            DYMU_FAIL(ctx, DYMU_ERR_ARG, "anisotropy table: entry %d is not a finite angle with a finite factor > 0", k);
+        if (k > 0 && !(theta_deg[k] > theta_deg[k - 1]))
+            DYMU_FAIL(ctx, DYMU_ERR_ARG, "anisotropy table: angles must be strictly ascending (entry %d)", k);
+    }
+    if (!ctx->dircost)
+        DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&ctx->dircost, 4 * (size_t)ctx->pitch * ctx->rows * sizeof(double)));
+    for (int k = 0; k < n; ++k)
+    {
+        ctx->aniso_theta[k] = theta_deg[k];
+        ctx->aniso_f[k] = factor[k];
+    }
+    ctx->aniso_n = n;
+    ctx->solved = false;
+    // a clean C_eff: build the planes now; otherwise the next refresh builds both
+    if (!ctx->ceff_dirty) DYMU_TRY(build_dircost(ctx));
+    return DYMU_OK;
+}
+
 int dymu_count_reached(dymu_ctx* ctx, uint32_t slot, uint64_t* n_finite)
 {
     DYMU_GUARD(ctx);
@@ -1009,6 +1129,32 @@ int dymu_internal_band_from_rows(dymu_ctx* ctx, uint32_t j0, uint32_t j1)
     return DYMU_OK;
 }
 
+// the directional-cost planes from elevation, C_eff and the table, and the band width of the
+// anisotropic solve (a few tile crossings worth of the mean directional cost)
+static int build_dircost(dymu_ctx* ctx)
+{
+    const size_t n = (size_t)ctx->pitch * ctx->rows;
+    AnisoTable tab;
+    tab.n = ctx->aniso_n;
+    for (int k = 0; k < DYMU_ANISO_MAX; ++k)
+    {
+        tab.theta[k] = k < tab.n ? ctx->aniso_theta[k] : 0.0;
+        tab.f[k] = k < tab.n ? ctx->aniso_f[k] : 0.0;
+    }
+    DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
+    double* d = (double*)ctx->d_scratch;
+    DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 16, ctx->stream));
+    k_dircost<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->elev, ctx->ceff, ctx->dircost, n, ctx->gres,
+                                                                 ctx->pitch, ctx->rows, ctx->nx, ctx->ny, tab, d);
+    ctx->launches++;
+    DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    double h[2] = {0, 0};
+    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->aniso_band = h[1] > 0 ? kBandFactor * (double)ctx->tile * (h[0] / h[1]) : 1.0 / 0.0;
+    return DYMU_OK;
+}
+
 int dymu_internal_refresh_ceff(dymu_ctx* ctx)
 {
     if (!ctx->ceff_dirty) return DYMU_OK;
@@ -1029,5 +1175,6 @@ int dymu_internal_refresh_ceff(dymu_ctx* ctx)
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->fim_band = h[1] > 0 ? kBandFactor * (double)ctx->tile * (h[0] / h[1]) : 1.0 / 0.0;
     ctx->ceff_dirty = false;
+    if (ctx->aniso_n) DYMU_TRY(build_dircost(ctx));
     return DYMU_OK;
 }

@@ -13,7 +13,9 @@ CUDA_SO = os.path.join(HERE, "libdymu_cuda.so")
 
 OK = 0
 PLANE = {"elevation": 0, "slope": 1, "raw_cost": 2, "cost": 3, "hazard_density": 4,
-         "trafficability": 5, "total_cost": 6, "ceff": 7}
+         "trafficability": 5, "total_cost": 6, "ceff": 7,
+         # directional costs of the anisotropic solve (read-only, only while it is on)
+         "dircost_xm": 8, "dircost_xp": 9, "dircost_ym": 10, "dircost_yp": 11}
 PLANE_U8 = {"obstacle": 0, "locmode": 1}
 XFORM_NONE, XFORM_INF_TO_MINUS1, XFORM_EFFECTIVE_COST = 0, 1, 2
 LPLANE = {"risk": 0, "deviation": 1, "total_cost": 2}
@@ -82,6 +84,7 @@ _SIG = {
                                         C.c_size_t, _dp, C.c_size_t]),
     "dymu_upload_terrain": (C.c_int, [C.c_void_p, _dp, C.c_size_t]),
     "dymu_reserve_slots": (C.c_int, [C.c_void_p, C.c_uint32]),
+    "dymu_set_anisotropy": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int]),
     "dymu_solve_total_cost": (C.c_int, [C.c_void_p, C.c_uint32, _u32p, _u32p,
                                         C.POINTER(SolveStats)]),
     "dymu_solve_start": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(SolveStats)]),
@@ -279,6 +282,14 @@ class DeviceLayer:
             n_locs, e.ctypes.data_as(_dp) if e is not None else None,
             e.shape[1] if e is not None else 0,
             t.ctypes.data_as(_dp) if t is not None else None, t.shape[1] if t is not None else 0))
+
+    def set_anisotropy(self, theta_deg, factors):
+        """Slope anisotropy: f(theta) piecewise linear in the table (theta in degrees, strictly
+        ascending, positive = uphill; factors finite > 0); empty tables switch it off."""
+        t, f = _f64(theta_deg).ravel(), _f64(factors).ravel()
+        if t.size != f.size:
+            raise ValueError("theta_deg and factors differ in length")
+        self._chk(self._l.dymu_set_anisotropy(self._h, t.ctypes.data_as(_dp), f.ctypes.data_as(_dp), t.size))
 
     # solve
     def reserve_slots(self, n):

@@ -60,6 +60,7 @@ _SIGNATURES = {
     "dymu_planner_set_total_cost_target": (C.c_int, [C.c_void_p, _dp, C.c_uint]),
     "dymu_planner_get_total_cost_matrix_flat": (C.c_int, [C.c_void_p, _dp, C.c_uint]),
     "dymu_planner_last_call_seconds": (C.c_double, [C.c_void_p]),
+    "dymu_planner_set_slope_anisotropy": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int]),
 }
 
 PLANNER_SYMBOLS = tuple(_SIGNATURES)
@@ -186,6 +187,13 @@ class Planner:
 
     def computeTotalCostMap(self, x, y):
         return bool(self._l.dymu_planner_compute_total_cost_map(self._h, x, y))
+
+    def setSlopeAnisotropy(self, slope_angles_deg, factors):
+        """Extension of the B200 drop-in (the reference build returns -1, reported as False)."""
+        a, f = _f64(slope_angles_deg).ravel(), _f64(factors).ravel()
+        if a.size != f.size:
+            return False
+        return self._l.dymu_planner_set_slope_anisotropy(self._h, _ptr(a), _ptr(f), a.size) == 1
 
     def computeEntireTotalCostMap(self):
         return bool(self._l.dymu_planner_compute_entire_total_cost_map(self._h))

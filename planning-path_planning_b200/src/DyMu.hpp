@@ -317,6 +317,13 @@ class DyMuPathPlanner
     // both maps to computeCostMap again.  With resolve=true and a goal set, the total-cost
     // map is recomputed as well.
     bool recomputeCostMap(bool resolve = false);
+    // Slope anisotropy for every later compute*TotalCostMap, getPath and computeGlobalPath: the
+    // cost of moving from a node to a 4-neighbour is its cost term times f(theta), theta the
+    // signed slope angle toward that neighbour in degrees (positive = uphill) and f piecewise
+    // linear in (slope_angles_deg, factors), clamped at both ends (DESIGN.md section 10).  Angles
+    // strictly ascending, factors finite > 0, at least two pairs; empty vectors switch it off.
+    // False before initGlobalLayer and on a malformed table.  The local layer stays isotropic.
+    bool setSlopeAnisotropy(const std::vector<double>& slope_angles_deg, const std::vector<double>& factors);
     // read-only view of the CoRa accumulators (test tap)
     const std::vector<segmentedTerrain>& terrainInfo() const { return terrain_vector; }
     // bulk tap of one globalNode field (DYMU_NODE_* of include/dymu_planner_c.h)

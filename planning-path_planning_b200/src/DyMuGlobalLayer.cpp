@@ -164,6 +164,15 @@ bool DyMuPathPlanner::setCostMap(const double* cost_map, size_t ld)
     return deviceOk(dymu_set_cost_map(dev, cost_map, ld), "setCostMap");
 }
 
+bool DyMuPathPlanner::setSlopeAnisotropy(const std::vector<double>& slope_angles_deg,
+                                         const std::vector<double>& factors)
+{
+    if (!dev || slope_angles_deg.size() != factors.size() || slope_angles_deg.size() > DYMU_ANISO_MAX) return false;
+    finishReadback();
+    return deviceOk(dymu_set_anisotropy(dev, slope_angles_deg.data(), factors.data(), (int)factors.size()),
+                    "setSlopeAnisotropy");
+}
+
 void DyMuPathPlanner::finishReadback()
 {
     if (readback_inflight && dev) deviceOk(dymu_download_total_cost_end(dev), "getTotalCostMatrix");
