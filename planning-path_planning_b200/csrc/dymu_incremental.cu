@@ -34,7 +34,7 @@ struct IncArgs
     const uint8_t* obst;
     double* ceff;
     double* T;
-    uint32_t pitch, rows, nx, ny, ntx, tile;
+    uint32_t pitch, rows, nx, ny, ntx, tile_edge;  // tile_edge = kTile (the kernels take it at run time)
     double gres;
     uint32_t goal_cell_lo, goal_cell_hi;  // padded-plane index of the goal, split (kept out of the cone)
     uint32_t* markbits;                   // one bit per padded cell
@@ -51,11 +51,11 @@ struct IncArgs
 __device__ __forceinline__ void wake_tile(const IncArgs& a, size_t q)
 {
     const uint32_t j = (uint32_t)(q / a.pitch), i = (uint32_t)(q % a.pitch);
-    const uint32_t t = (j / a.tile) * a.ntx + i / a.tile;
+    const uint32_t t = (j / a.tile_edge) * a.ntx + i / a.tile_edge;
     if (atomicOr(&a.flag0[t], kFullTile) == 0)
     {
         a.key0[t] = 0ull;
-        a.list0[atomicAdd(&a.ctrl[0], 1u)] = t;
+        a.list0[atomicAdd(&a.ctrl[kCtrlCount], 1u)] = t;
         a.gmin[0] = 0ull;
     }
 }
@@ -195,9 +195,7 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
     }
     ctx->export_done = false;
     dymu_fim_work* w = &ctx->work;
-    DYMU_TRY(dymu_internal_fim_reset(ctx, w));
-    w->rot = 0;
-    w->pending = false;
+    DYMU_TRY(dymu_internal_fim_clear(ctx, w));  // k_inc_diff / k_inc_apply queue the tiles
     DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
     uint32_t* d_cnt = (uint32_t*)ctx->d_scratch;
     DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d_cnt, 0, 16, ctx->stream));
@@ -205,7 +203,7 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
     IncArgs a;
     a.cost = ctx->cost; a.haz = ctx->haz; a.traff = ctx->traff; a.obst = ctx->obst; a.ceff = ctx->ceff;
     a.T = ctx->T; a.pitch = ctx->pitch; a.rows = ctx->rows; a.nx = ctx->nx; a.ny = ctx->ny;
-    a.ntx = ctx->ntx; a.tile = ctx->tile; a.gres = ctx->gres;
+    a.ntx = ctx->ntx; a.tile_edge = kTile; a.gres = ctx->gres;
     const size_t goal = (size_t)goal_j * ctx->pitch + goal_i;
     a.goal_cell_lo = (uint32_t)goal; a.goal_cell_hi = (uint32_t)(goal >> 32);
     a.markbits = ctx->inc_markbits; a.visited = ctx->inc_visited; a.cap = ctx->inc_cap; a.counters = d_cnt;
@@ -243,15 +241,10 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
         ctx->launches++;
         DYMU_CUDA_TRY(ctx, cudaGetLastError());
     }
-    dymu_fim_launch L;
-    L.T = ctx->T; L.slot_stride = n; L.C = ctx->ceff; L.pitch = ctx->pitch; L.rows = ctx->rows;
-    L.ntx = ctx->ntx; L.nty = ctx->nty; L.nprob = 1; L.mode = 0; L.tile = (int)ctx->tile;
-    L.work = w; L.n_initial = 0; L.band = ctx->fim_band; L.seed_kind = 3; L.seed_data = nullptr;
-    L.preseeded = true;
     dymu_solve_stats local;
     memset(&local, 0, sizeof(local));
     ctx->solved = false;
-    int rc = dymu_internal_fim_run(ctx, L, &local);
+    int rc = dymu_internal_fim_run(ctx, dymu_internal_global_launch(ctx, 1), &local);
     if (rc == DYMU_OK || rc == DYMU_ERR_NOCONV)
     {
         cudaEventElapsedTime(&local.reset_ms, ctx->ev0, ctx->ev1);  // diff + marking + invalidation

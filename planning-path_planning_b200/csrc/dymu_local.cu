@@ -1120,8 +1120,7 @@ static int local_alloc(dymu_ctx* ctx, dymu_local& l, uint32_t wg)
     if (l.r < 1) DYMU_FAIL(ctx, DYMU_ERR_ARG, "local_res must not exceed global_res");
     if ((uint64_t)wg * l.r > 65535u) DYMU_FAIL(ctx, DYMU_ERR_ARG, "local window of %u nodes is too large", wg);
     l.w = wg * l.r;
-    uint32_t tile = ctx->tile;
-    l.pitch = dymu_div_up(l.w, tile) * tile;
+    l.pitch = dymu_div_up(l.w, kTile) * kTile;
     l.rows = l.pitch;
     size_t n = (size_t)l.pitch * l.rows;
     double** f64[] = {&l.risk, &l.dev, &l.ltot, &l.crisk};
@@ -1136,7 +1135,7 @@ static int local_alloc(dymu_ctx* ctx, dymu_local& l, uint32_t wg)
     DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&l.entered, (size_t)wg * wg));
     DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&l.axis_d2, (size_t)2 * l.w * sizeof(double)));
     DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&l.axis_node, (size_t)2 * wg * sizeof(int32_t)));
-    uint32_t nt = l.pitch / tile;
+    uint32_t nt = l.pitch / kTile;
     DYMU_TRY(dymu_internal_fim_alloc(ctx, &l.work, (size_t)nt * nt));
     l.allocated = true;
     return DYMU_OK;
@@ -1394,13 +1393,12 @@ int dymu_local_expand_risk(dymu_ctx* ctx, double risk_distance, dymu_solve_stats
                                                  l.rows, l.w);
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
-    uint32_t nt = l.pitch / ctx->tile;
+    uint32_t nt = l.pitch / kTile;
+    DYMU_TRY(dymu_internal_fim_seed_all(ctx, &l.work, nt * nt));
     dymu_fim_launch L;
     L.T = l.risk; L.slot_stride = n; L.C = l.crisk; L.pitch = l.pitch; L.rows = l.rows;
-    L.ntx = nt; L.nty = nt; L.nprob = 1; L.mode = 1; L.tile = (int)ctx->tile; L.work = &l.work;
-    L.n_initial = nt * nt;
+    L.ntx = nt; L.nty = nt; L.nprob = 1; L.mode = 1; L.work = &l.work;
     L.band = 1.0 / 0.0;  // small window: plain FIM
-    L.seed_kind = 2; L.seed_data = nullptr;
     DYMU_TRY(dymu_internal_fim_run(ctx, L, stats));
     k_mark_entered_risk<<<grid, 256, 0, ctx->stream>>>(make_view(ctx), l.entered);
     ctx->launches++;

@@ -501,11 +501,10 @@ int dymu_create(int device, uint32_t nx, uint32_t ny, double global_res, double 
     ctx->ny = ny;
     ctx->gres = global_res;
     ctx->lres = local_res;
-    ctx->tile = 32;
-    ctx->ntx = dymu_div_up(nx, ctx->tile);
-    ctx->nty = dymu_div_up(ny, ctx->tile);
-    ctx->pitch = ctx->ntx * ctx->tile;
-    ctx->rows = ctx->nty * ctx->tile;
+    ctx->ntx = dymu_div_up(nx, kTile);
+    ctx->nty = dymu_div_up(ny, kTile);
+    ctx->pitch = ctx->ntx * kTile;
+    ctx->rows = ctx->nty * kTile;
     ctx->n_slots = 1;
     *out = ctx;  // from here on the caller owns ctx and can read the error text
     DYMU_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
@@ -614,7 +613,7 @@ int dymu_event_elapsed_ms(dymu_ctx* ctx, int a, int b, float* ms)
 int dymu_geometry(const dymu_ctx* ctx, uint32_t* tile, uint32_t* pitch, uint32_t* rows)
 {
     if (!ctx) return DYMU_ERR_ARG;
-    if (tile) *tile = ctx->tile;
+    if (tile) *tile = kTile;
     if (pitch) *pitch = ctx->pitch;
     if (rows) *rows = ctx->rows;
     return DYMU_OK;
@@ -1125,7 +1124,7 @@ int dymu_internal_band_from_rows(dymu_ctx* ctx, uint32_t j0, uint32_t j1)
     double h[2] = {0, 0};
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (h[1] > 0) ctx->fim_band = kBandFactor * (double)ctx->tile * (h[0] / h[1]);
+    if (h[1] > 0) ctx->fim_band = kBandFactor * (double)kTile * (h[0] / h[1]);
     return DYMU_OK;
 }
 
@@ -1151,7 +1150,7 @@ static int build_dircost(dymu_ctx* ctx)
     double h[2] = {0, 0};
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->aniso_band = h[1] > 0 ? kBandFactor * (double)ctx->tile * (h[0] / h[1]) : 1.0 / 0.0;
+    ctx->aniso_band = h[1] > 0 ? kBandFactor * (double)kTile * (h[0] / h[1]) : 1.0 / 0.0;
     return DYMU_OK;
 }
 
@@ -1173,7 +1172,7 @@ int dymu_internal_refresh_ceff(dymu_ctx* ctx)
     double h[2] = {0, 0};
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->fim_band = h[1] > 0 ? kBandFactor * (double)ctx->tile * (h[0] / h[1]) : 1.0 / 0.0;
+    ctx->fim_band = h[1] > 0 ? kBandFactor * (double)kTile * (h[0] / h[1]) : 1.0 / 0.0;
     ctx->ceff_dirty = false;
     if (ctx->aniso_n) DYMU_TRY(build_dircost(ctx));
     return DYMU_OK;
