@@ -56,6 +56,9 @@ typedef struct dymu_ctx dymu_ctx;
 #define DYMU_PLANE_DIRCOST_XP 9
 #define DYMU_PLANE_DIRCOST_YM 10
 #define DYMU_PLANE_DIRCOST_YP 11
+/* distance in metres from a cell to the nearest obstacle cell, +inf beyond radius + margin (see
+ * dymu_set_obstacle_clearance).  Read-only; it exists only while obstacle clearance is on. */
+#define DYMU_PLANE_CLEARANCE 12
 /* byte / word planes */
 #define DYMU_PLANE_U8_OBSTACLE 0
 #define DYMU_PLANE_U8_LOCMODE 1 /* index into locomotion_modes, 255 = "DONT_CARE" */
@@ -153,6 +156,7 @@ int dymu_upload_terrain(dymu_ctx* ctx, const double* terrain, size_t ld);
  * for theta_deg[k] <= theta < theta_deg[k+1].  For a cell x and its 4-neighbour m
  *     theta(x->m) = atan((elev[m]-elev[x]) / global_res) * (180/pi)
  *     a(x->m)     = C_eff(x) * f(theta(x->m))      (C_eff: DYMU_PLANE_CEFF; +inf toward outside)
+ * (with obstacle clearance on, C_eff is the clearance-adjusted one)
  * and the total-cost update of x is the smallest of the four one-sided values T[m] + a(x->m)
  * and, for each pair (h in {i-1,i+1}, v in {j-1,j+1}) with -a_h < T_h - T_v < a_v, the root
  *     ((a_v^2*T_h + a_h^2*T_v) + (a_h*a_v)*sqrt((a_h^2+a_v^2) - d^2)) / (a_h^2+a_v^2),  d = T_h-T_v.
@@ -164,6 +168,35 @@ int dymu_upload_terrain(dymu_ctx* ctx, const double* terrain, size_t ld);
  * the directional-cost planes; any other malformed table is DYMU_ERR_ARG. */
 #define DYMU_ANISO_MAX 64
 int dymu_set_anisotropy(dymu_ctx* ctx, const double* theta_deg, const double* factor, int n);
+
+/* ---- obstacle clearance (an extension; the reference plans for a point) ---------------------
+ * radius, margin, penalty: finite, >= 0, metres (penalty: dimensionless).  With g = global_res and
+ * R = floor((radius + margin) / g) <= DYMU_CLEARANCE_MAX_CELLS, let s(x) be the smallest
+ * di*di + dj*dj over obstacle cells (i+di, j+dj) with |di| <= R and |dj| <= R (cells outside the grid
+ * are not obstacles).  The clearance is d(x) = sqrt(s) * g, +inf when there is no such obstacle or
+ * d > radius + margin (= distance_transform_edt of the free cells times g, cut off there).  With c the
+ * plain cost term (DYMU_PLANE_CEFF without clearance), C_eff becomes
+ *     +inf                                                 on obstacles and for d <= radius (lethal ring)
+ *     c * (1.0 + penalty * ((radius + margin - d) / margin))  for radius < d < radius + margin
+ *     c                                                    otherwise
+ * Lethal-ring cells are never propagation targets, like obstacles, but the obstacle plane stays as it
+ * is.  So a goal inside the ring is not a valid goal: the solve still seeds it (only goals on obstacle
+ * cells are refused), but the planner class rejects it as it rejects a goal on an obstacle.  A start
+ * inside the ring has no finite total cost, like a start on an obstacle.  Every
+ * solve reads the adjusted C_eff: dymu_solve_total_cost (any slot count), dymu_solve_incremental
+ * (still incremental), dymu_solve_start / _advance on a whole grid, dymu_batch_solve, direct delivery,
+ * the path extraction and, through the directional costs, slope anisotropy.  dymu_plan_streamed and a
+ * streamed dymu_set_cost_map_begin complete the upload first and then run the full solve (clearance
+ * near a seam needs rows that have not arrived yet).  dymu_dd_solve returns DYMU_ERR_STATE when any
+ * strip has clearance on (a strip cannot see obstacles across a cut); a phase-bounded solve on a
+ * strip sees only that strip's obstacles.  The clearance plane is rebuilt only when the obstacle
+ * plane changed (dymu_set_cost_map, dymu_compute_cost_map, a streamed upload); changes of cost,
+ * hazard_density or trafficability only re-run the C_eff pass.  radius == 0 && margin == 0 switches
+ * it off and frees its planes; a negative, NaN or infinite value, or R > DYMU_CLEARANCE_MAX_CELLS, is
+ * DYMU_ERR_ARG.  While it is off, DYMU_PLANE_CLEARANCE is an unknown plane (DYMU_ERR_ARG).  Any
+ * change marks the resident total-cost map as stale. */
+#define DYMU_CLEARANCE_MAX_CELLS 128
+int dymu_set_obstacle_clearance(dymu_ctx* ctx, double radius, double margin, double penalty);
 
 /* ---- total-cost solve -------------------------------------------------------- */
 /* Number of independent total-cost planes ("slots") for batched goal queries. */

@@ -155,6 +155,10 @@ int dymu_planner_get_total_cost_matrix_flat(dymu_planner* p, double* out, unsign
  * angle in degrees and cost factor, n = 0 switches it off; 1 = applied, 0 = rejected.  The
  * reference has no such capability: its build returns -1. */
 int dymu_planner_set_slope_anisotropy(dymu_planner* p, const double* angles, const double* factors, int n);
+/* setObstacleClearance(radius, margin, penalty) (extension of the B200 drop-in, metres): lethal
+ * radius and penalised margin around obstacle nodes, radius = margin = 0 switches it off; 1 = applied,
+ * 0 = rejected.  The reference has no such capability: its build returns -1. */
+int dymu_planner_set_obstacle_clearance(dymu_planner* p, double radius, double margin, double penalty);
 
 double dymu_planner_last_call_seconds(dymu_planner* p);
 

@@ -451,6 +451,20 @@ int dymu_planner_set_slope_anisotropy(dymu_planner* p, const double* angles, con
 #endif
 }
 
+int dymu_planner_set_obstacle_clearance(dymu_planner* p, double radius, double margin, double penalty)
+{
+    if (!p) return -1;
+#if defined(DYMU_CAPI_B200)
+    Stopwatch sw(&p->last_seconds);
+    return p->impl->setObstacleClearance(radius, margin, penalty) ? 1 : 0;
+#else
+    (void)radius;
+    (void)margin;
+    (void)penalty;
+    return -1;  // the reference plans for a point
+#endif
+}
+
 int dymu_planner_set_cost_map_flat(dymu_planner* p, const double* cost, unsigned ld)
 {
     if (!p || !cost || ld < p->nx) return -1;

@@ -1381,8 +1381,9 @@ int dymu_solve_total_cost(dymu_ctx* ctx, uint32_t n_goals, const uint32_t* goal_
     if (ctx && ctx->upload_pending)
     {
         // a cost map is still on its way (dymu_set_cost_map_begin): start on the rows that are there
-        // (the anisotropic solve waits for the whole map: its directional costs need every row)
-        if (!ctx->aniso_n && n_goals == 1 && goal_i && goal_j && goal_i[0] < ctx->nx && goal_j[0] >= ctx->up_a0
+        // (the anisotropic solve waits for the whole map: its directional costs need every row; so
+        // does obstacle clearance, which near a seam needs obstacles of rows still on their way)
+        if (!ctx->aniso_n && !ctx->clear_on && n_goals == 1 && goal_i && goal_j && goal_i[0] < ctx->nx && goal_j[0] >= ctx->up_a0
             && goal_j[0] < ctx->up_a1)
             return solve_streamed(ctx, goal_i[0], goal_j[0], 0, stats);
         DYMU_TRY(dymu_internal_settle_upload(ctx));
@@ -1657,9 +1658,9 @@ int dymu_plan_streamed(dymu_ctx* ctx, const double* cost_host, size_t ld, uint32
     DYMU_GUARD_ONLY(ctx);
     if (!ctx || !cost_host || ld < ctx->nx || goal_i >= ctx->nx || goal_j >= ctx->ny) return DYMU_ERR_ARG;
     DYMU_TRY(dymu_set_cost_map_begin(ctx, cost_host, ld, goal_j));
-    if (ctx->aniso_n)
+    if (ctx->aniso_n || ctx->clear_on)
     {
-        // the directional costs need the whole map: upload first, then the full solve
+        // the directional costs and the clearance need the whole map: upload first, then the full solve
         DYMU_TRY(dymu_internal_settle_upload(ctx));
         return solve_total_cost_impl(ctx, 1, &goal_i, &goal_j, 0, 0, stats);
     }

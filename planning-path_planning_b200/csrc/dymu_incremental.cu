@@ -19,6 +19,10 @@
 //   3. k_inc_apply  marked cells go back to +inf, their tiles are queued.
 //   4. the tile FIM kernel runs from that seeded state.
 //
+// With obstacle clearance on, step 1 applies the clearance adjustment (dymu_clearance_ceff) to the
+// resident clearance plane, rebuilt first if the obstacles changed.  The update stays monotone and
+// upwind, so a cell whose adjusted C went up is a cone root like any other.
+//
 // The result is the fixed point of propagateGlobalNode (G.cpp:500-546) for the new planes, i.e.
 // what a full solve gives, to rounding.  When the cone outgrows its buffer the call falls back to
 // the full solve.
@@ -60,7 +64,15 @@ __device__ __forceinline__ void wake_tile(const IncArgs& a, size_t q)
     }
 }
 
-__global__ void k_inc_diff(IncArgs a)
+// the clearance adjustment of k_inc_diff<true> (dymu_set_obstacle_clearance)
+struct IncClear
+{
+    const double* clear;
+    double radius, margin, penalty;
+};
+
+template <bool kClear>
+__global__ void k_inc_diff(IncArgs a, IncClear cl)
 {
     const size_t total = (size_t)a.pitch * a.rows;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
@@ -69,7 +81,11 @@ __global__ void k_inc_diff(IncArgs a)
     {
         const uint32_t j = (uint32_t)(q / a.pitch), i = (uint32_t)(q % a.pitch);
         double c = DYMU_INF;
-        if (i < a.nx && j < a.ny && !a.obst[q]) c = a.gres * (a.cost[q]) * (2 + a.haz[q] - a.traff[q]);
+        if (i < a.nx && j < a.ny && !a.obst[q])
+        {
+            c = a.gres * (a.cost[q]) * (2 + a.haz[q] - a.traff[q]);
+            if (kClear) c = dymu_clearance_ceff(c, cl.clear[q], cl.radius, cl.margin, cl.penalty);
+        }
         const double old = a.ceff[q];
         if (c == old) continue;
         a.ceff[q] = c;
@@ -196,6 +212,7 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
     ctx->export_done = false;
     dymu_fim_work* w = &ctx->work;
     DYMU_TRY(dymu_internal_fim_clear(ctx, w));  // k_inc_diff / k_inc_apply queue the tiles
+    DYMU_TRY(dymu_internal_clearance_update(ctx));  // the obstacles may have changed
     DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
     uint32_t* d_cnt = (uint32_t*)ctx->d_scratch;
     DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d_cnt, 0, 16, ctx->stream));
@@ -211,7 +228,11 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
     int grid = (int)((n + 255) / 256);
     if (grid > ctx->sm_count * 16) grid = ctx->sm_count * 16;
     DYMU_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    k_inc_diff<<<grid, 256, 0, ctx->stream>>>(a);
+    if (ctx->clear_on)
+        k_inc_diff<true><<<grid, 256, 0, ctx->stream>>>(
+            a, IncClear{ctx->clear, ctx->clear_radius, ctx->clear_margin, ctx->clear_penalty});
+    else
+        k_inc_diff<false><<<grid, 256, 0, ctx->stream>>>(a, IncClear{});
     k_inc_mark<<<1, 1024, 0, ctx->stream>>>(a);
     ctx->launches += 2;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());

@@ -245,6 +245,8 @@ int dymu_dd_solve(dymu_ctx** ctxs, uint32_t n, const uint32_t* cuts, uint32_t go
         if (!ctxs[k]->have_cost) DYMU_FAIL(ctxs[k], DYMU_ERR_STATE, "strip %u has no cost map", k);
         if (ctxs[k]->aniso_n)
             DYMU_FAIL(ctxs[k], DYMU_ERR_STATE, "strip %u: domain decomposition is isotropic only", k);
+        if (ctxs[k]->clear_on)
+            DYMU_FAIL(ctxs[k], DYMU_ERR_STATE, "strip %u: a strip cannot see obstacles across a cut (obstacle clearance)", k);
     }
     if (goal_i >= ctxs[0]->nx || goal_j < cuts[0] || goal_j >= cuts[n]) return DYMU_ERR_ARG;
     DdShared S;

@@ -415,6 +415,7 @@ double* plane_ptr(dymu_ctx* ctx, int plane)
             // only while anisotropy is on
             return ctx->dircost ? ctx->dircost + (size_t)(plane - DYMU_PLANE_DIRCOST_XM) * ctx->pitch * ctx->rows
                                 : nullptr;
+        case DYMU_PLANE_CLEARANCE: return ctx->clear;  // only while obstacle clearance is on
         default: return nullptr;
     }
 }
@@ -437,6 +438,17 @@ int fill_plane(dymu_ctx* ctx, double* p, double v, size_t n)
 }
 
 bool is_dircost(int plane) { return plane >= DYMU_PLANE_DIRCOST_XM && plane <= DYMU_PLANE_DIRCOST_YP; }
+// planes derived from the others on the device, never written from outside
+bool is_read_only(int plane) { return is_dircost(plane) || plane == DYMU_PLANE_CLEARANCE; }
+
+// brings a derived plane up to date before it is read
+int refresh_for_read(dymu_ctx* ctx, int plane)
+{
+    if (plane == DYMU_PLANE_CEFF || is_dircost(plane)) return dymu_internal_refresh_ceff(ctx);
+    // the clearance plane alone: C_eff stays dirty for dymu_solve_incremental to compare against
+    if (plane == DYMU_PLANE_CLEARANCE) return dymu_internal_clearance_update(ctx);
+    return DYMU_OK;
+}
 
 // planes C_eff (and, while anisotropy is on, the directional costs) are built from
 bool feeds_ceff(const dymu_ctx* ctx, int plane)
@@ -553,6 +565,7 @@ int dymu_destroy(dymu_ctx* ctx)
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     dymu_internal_local_free(ctx);
     dymu_internal_incremental_free(ctx);
+    dymu_internal_clearance_free(ctx);
     dymu_internal_fim_free(&ctx->work);
     void* ptrs[] = {ctx->elev, ctx->slope, ctx->raw, ctx->cost, ctx->haz, ctx->traff, ctx->ceff,
                     ctx->T, ctx->terrain, ctx->obst, ctx->locmode, ctx->d_lut, ctx->d_slopes,
@@ -624,6 +637,7 @@ int dymu_upload_plane(dymu_ctx* ctx, int plane, const double* host, size_t ld)
     DYMU_GUARD(ctx);
     if (!ctx || !host || ld < ctx->nx) return DYMU_ERR_ARG;
     if (is_dircost(plane)) DYMU_FAIL(ctx, DYMU_ERR_ARG, "the directional-cost planes are read-only");
+    if (plane == DYMU_PLANE_CLEARANCE) DYMU_FAIL(ctx, DYMU_ERR_ARG, "the clearance plane is read-only");
     double* d = plane_ptr(ctx, plane);
     if (!d) DYMU_FAIL(ctx, DYMU_ERR_ARG, "unknown plane %d", plane);
     if (plane == DYMU_PLANE_TOTAL_COST) DYMU_TRY(dymu_internal_settle_delivery(ctx));
@@ -686,7 +700,7 @@ int dymu_download_plane(dymu_ctx* ctx, int plane, double* host, size_t ld, int x
 {
     DYMU_GUARD(ctx);
     if (!ctx || !host || ld < ctx->nx) return DYMU_ERR_ARG;
-    if (plane == DYMU_PLANE_CEFF || is_dircost(plane)) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
+    DYMU_TRY(refresh_for_read(ctx, plane));
     double* d = plane_ptr(ctx, plane);
     if (!d) DYMU_FAIL(ctx, DYMU_ERR_ARG, "unknown plane %d", plane);
     return download_f64(ctx, d, host, ld, xform);
@@ -787,7 +801,7 @@ int dymu_read_rect(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32_t 
 {
     DYMU_GUARD(ctx);
     if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h)) return DYMU_ERR_ARG;
-    if (plane == DYMU_PLANE_CEFF || is_dircost(plane)) DYMU_TRY(dymu_internal_refresh_ceff(ctx));
+    DYMU_TRY(refresh_for_read(ctx, plane));
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     DYMU_CUDA_TRY(ctx, cudaMemcpy2DAsync(host, w * sizeof(double), d + (size_t)j0 * ctx->pitch + i0,
@@ -801,7 +815,7 @@ int dymu_write_rect(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32_t
                     const double* host)
 {
     DYMU_GUARD(ctx);
-    if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h) || is_dircost(plane)) return DYMU_ERR_ARG;
+    if (!ctx || !host || !rect_ok(ctx, i0, j0, w, h) || is_read_only(plane)) return DYMU_ERR_ARG;
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     if (plane == DYMU_PLANE_TOTAL_COST) DYMU_TRY(dymu_internal_settle_delivery(ctx));
@@ -831,7 +845,7 @@ int dymu_read_rect_u8(dymu_ctx* ctx, int plane, uint32_t i0, uint32_t j0, uint32
 int dymu_plane_device_ptr(dymu_ctx* ctx, int plane, void** dptr, size_t* pitch_elems)
 {
     DYMU_GUARD(ctx);
-    if (!ctx || !dptr || is_dircost(plane)) return DYMU_ERR_ARG;
+    if (!ctx || !dptr || is_read_only(plane)) return DYMU_ERR_ARG;
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     *dptr = d;
@@ -856,6 +870,7 @@ int dymu_set_cost_map(dymu_ctx* ctx, const double* host, size_t ld)
         ctx->cost, ctx->obst, ctx->traff, ctx->haz, ctx->pitch, ctx->nx, ctx->ny);
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    ctx->obst_epoch++;
     ctx->have_cost = true;
     ctx->ceff_dirty = true;
     return DYMU_OK;
@@ -920,6 +935,7 @@ int dymu_compute_cost_map(dymu_ctx* ctx, const double* cost_lut, int n_lut, cons
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));  // cost_lut/slopes are caller memory
     ctx->terrain_staged = false;
     ctx->have_terrain = true;
+    ctx->obst_epoch++;
     ctx->have_cost = true;
     ctx->ceff_dirty = true;
     return DYMU_OK;
@@ -963,6 +979,9 @@ int dymu_time_stencils(dymu_ctx* ctx, float ms[6])
         ctx->launches += 4;
     }
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    ctx->obst_epoch++;  // k_set_cost_map wrote the obstacle plane (with the values it already held)
+    // k_ceff wrote the plain cost term: put the clearance-adjusted C_eff back (the band width stays)
+    if (ctx->clear_on && !ctx->ceff_dirty) DYMU_TRY(dymu_internal_clearance_ceff(ctx, nullptr));
     return DYMU_OK;
 }
 
@@ -972,6 +991,7 @@ int dymu_read_cells(dymu_ctx* ctx, int plane, uint32_t slot, const uint32_t* cel
     DYMU_GUARD(ctx);
     if (!ctx || !cell_index || !out) return DYMU_ERR_ARG;
     if (n == 0) return DYMU_OK;
+    if (plane == DYMU_PLANE_CLEARANCE) DYMU_TRY(dymu_internal_clearance_update(ctx));
     double* d = plane_ptr(ctx, plane);
     if (!d) return DYMU_ERR_ARG;
     if (plane == DYMU_PLANE_TOTAL_COST)
@@ -1087,6 +1107,7 @@ int dymu_internal_cost_rows(dymu_ctx* ctx, uint32_t j0, uint32_t j1)
         ctx->cost + off, ctx->obst + off, ctx->traff + off, ctx->haz + off, ctx->pitch, ctx->nx, nr);
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    ctx->obst_epoch++;
     k_ceff<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->cost + off, ctx->haz + off, ctx->traff + off,
                                                              ctx->obst + off, ctx->ceff + off, ctx->gres,
                                                              ctx->pitch, nr, ctx->nx, nr, nullptr);
@@ -1105,6 +1126,7 @@ int dymu_internal_settle_upload(dymu_ctx* ctx)
         ctx->cost, ctx->obst, ctx->traff, ctx->haz, ctx->pitch, ctx->nx, ctx->ny);
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    ctx->obst_epoch++;
     ctx->have_cost = true;
     ctx->ceff_dirty = true;
     return DYMU_OK;
@@ -1163,12 +1185,16 @@ int dymu_internal_refresh_ceff(dymu_ctx* ctx)
     DYMU_TRY(dymu_internal_scratch(ctx, 64, 64));
     double* d = (double*)ctx->d_scratch;
     DYMU_CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 16, ctx->stream));
-    k_ceff<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->cost, ctx->haz, ctx->traff,
-                                                             ctx->obst, ctx->ceff, ctx->gres,
-                                                             ctx->pitch, ctx->rows, ctx->nx,
-                                                             ctx->ny, d);
-    ctx->launches++;
-    DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    if (ctx->clear_on) DYMU_TRY(dymu_internal_clearance_ceff(ctx, d));
+    else
+    {
+        k_ceff<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->cost, ctx->haz, ctx->traff,
+                                                                 ctx->obst, ctx->ceff, ctx->gres,
+                                                                 ctx->pitch, ctx->rows, ctx->nx,
+                                                                 ctx->ny, d);
+        ctx->launches++;
+        DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    }
     double h[2] = {0, 0};
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));

@@ -15,7 +15,9 @@ OK = 0
 PLANE = {"elevation": 0, "slope": 1, "raw_cost": 2, "cost": 3, "hazard_density": 4,
          "trafficability": 5, "total_cost": 6, "ceff": 7,
          # directional costs of the anisotropic solve (read-only, only while it is on)
-         "dircost_xm": 8, "dircost_xp": 9, "dircost_ym": 10, "dircost_yp": 11}
+         "dircost_xm": 8, "dircost_xp": 9, "dircost_ym": 10, "dircost_yp": 11,
+         # distance to the nearest obstacle (read-only, only while obstacle clearance is on)
+         "clearance": 12}
 PLANE_U8 = {"obstacle": 0, "locmode": 1}
 XFORM_NONE, XFORM_INF_TO_MINUS1, XFORM_EFFECTIVE_COST = 0, 1, 2
 LPLANE = {"risk": 0, "deviation": 1, "total_cost": 2}
@@ -85,6 +87,7 @@ _SIG = {
     "dymu_upload_terrain": (C.c_int, [C.c_void_p, _dp, C.c_size_t]),
     "dymu_reserve_slots": (C.c_int, [C.c_void_p, C.c_uint32]),
     "dymu_set_anisotropy": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int]),
+    "dymu_set_obstacle_clearance": (C.c_int, [C.c_void_p, C.c_double, C.c_double, C.c_double]),
     "dymu_solve_total_cost": (C.c_int, [C.c_void_p, C.c_uint32, _u32p, _u32p,
                                         C.POINTER(SolveStats)]),
     "dymu_solve_start": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(SolveStats)]),
@@ -290,6 +293,11 @@ class DeviceLayer:
         if t.size != f.size:
             raise ValueError("theta_deg and factors differ in length")
         self._chk(self._l.dymu_set_anisotropy(self._h, t.ctypes.data_as(_dp), f.ctypes.data_as(_dp), t.size))
+
+    def set_obstacle_clearance(self, radius, margin, penalty):
+        """Obstacle clearance (metres): C_eff = +inf within `radius` of an obstacle, scaled by
+        1 + penalty * (radius + margin - d) / margin up to radius + margin; (0, 0, 0) switches it off."""
+        self._chk(self._l.dymu_set_obstacle_clearance(self._h, float(radius), float(margin), float(penalty)))
 
     # solve
     def reserve_slots(self, n):

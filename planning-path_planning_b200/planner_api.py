@@ -61,6 +61,7 @@ _SIGNATURES = {
     "dymu_planner_get_total_cost_matrix_flat": (C.c_int, [C.c_void_p, _dp, C.c_uint]),
     "dymu_planner_last_call_seconds": (C.c_double, [C.c_void_p]),
     "dymu_planner_set_slope_anisotropy": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int]),
+    "dymu_planner_set_obstacle_clearance": (C.c_int, [C.c_void_p, C.c_double, C.c_double, C.c_double]),
 }
 
 PLANNER_SYMBOLS = tuple(_SIGNATURES)
@@ -194,6 +195,12 @@ class Planner:
         if a.size != f.size:
             return False
         return self._l.dymu_planner_set_slope_anisotropy(self._h, _ptr(a), _ptr(f), a.size) == 1
+
+    def setObstacleClearance(self, radius, margin, penalty):
+        """Extension of the B200 drop-in: lethal radius and penalised margin around obstacles (metres);
+        (0, 0, 0) switches it off.  The reference build returns -1, reported as False."""
+        return self._l.dymu_planner_set_obstacle_clearance(self._h, float(radius), float(margin),
+                                                           float(penalty)) == 1
 
     def computeEntireTotalCostMap(self):
         return bool(self._l.dymu_planner_compute_entire_total_cost_map(self._h))

@@ -139,6 +139,7 @@ class DyMuPathPlanner
     size_t readback_ld;
     bool readback_inflight;
     bool streamed_cost;  // the last cost-map call was a streamed setCostMap(const double*, ld)
+    double clearance_radius;  // lethal radius of the obstacle clearance in effect (0: none)
     // obstacles ingested but not yet expanded (local_expandable_obstacles, DyMu.hpp:452)
     bool pending_risk;
     uint local_window_nodes;
@@ -159,6 +160,7 @@ class DyMuPathPlanner
     bool ensureLocalWindow(double x, double y, double half_x, double half_y, bool may_grow);
     bool growLocalWindow(long lo_x, long hi_x, long lo_y, long hi_y);
     bool readNode(uint i, uint j, globalNode& out);
+    bool goalInLethalRing();
     void markEntered();
     long localPropagationCell(base::Waypoint wInit, base::Waypoint wOvertake);
     std::vector<base::Waypoint> localPathFromCell(long cell, base::Waypoint wInit);
@@ -324,6 +326,15 @@ class DyMuPathPlanner
     // strictly ascending, factors finite > 0, at least two pairs; empty vectors switch it off.
     // False before initGlobalLayer and on a malformed table.  The local layer stays isotropic.
     bool setSlopeAnisotropy(const std::vector<double>& slope_angles_deg, const std::vector<double>& factors);
+    // Obstacle clearance for every later compute*TotalCostMap, getPath and computeGlobalPath (metres;
+    // DESIGN.md section 11): nodes within `radius` of an obstacle node become impassable (the lethal
+    // ring; the obstacle map itself is unchanged), the cost of nodes between radius and
+    // radius + margin is scaled by 1 + penalty * (radius + margin - d) / margin, d the distance to the
+    // nearest obstacle node.  radius = margin = 0 switches it off.  A goal inside the lethal ring is
+    // not valid, like a goal on an obstacle.  False before initGlobalLayer and on a malformed setting
+    // (negative or non-finite values, radius + margin over 128 global nodes).  The local layer keeps
+    // its own risk dilation.
+    bool setObstacleClearance(double radius, double margin, double penalty);
     // read-only view of the CoRa accumulators (test tap)
     const std::vector<segmentedTerrain>& terrainInfo() const { return terrain_vector; }
     // bulk tap of one globalNode field (DYMU_NODE_* of include/dymu_planner_c.h)

@@ -50,6 +50,7 @@ DyMuPathPlanner::DyMuPathPlanner(double risk_distance,
       readback_ld(0),
       readback_inflight(false),
       streamed_cost(false),
+      clearance_radius(0.0),
       pending_risk(false),
       local_window_nodes(64),
       local_ready(false),
@@ -118,6 +119,7 @@ bool DyMuPathPlanner::initGlobalLayer(double globalres,
     goal_set = false;
     global_goal = NULL;
     closed_threshold = kInf;
+    clearance_radius = 0.0;
     pending_risk = false;
     local_ready = false;
     // the local window is allocated up front (the reference builds its whole node graph here): the
@@ -171,6 +173,26 @@ bool DyMuPathPlanner::setSlopeAnisotropy(const std::vector<double>& slope_angles
     finishReadback();
     return deviceOk(dymu_set_anisotropy(dev, slope_angles_deg.data(), factors.data(), (int)factors.size()),
                     "setSlopeAnisotropy");
+}
+
+bool DyMuPathPlanner::setObstacleClearance(double radius, double margin, double penalty)
+{
+    if (!dev) return false;
+    finishReadback();
+    if (!deviceOk(dymu_set_obstacle_clearance(dev, radius, margin, penalty), "setObstacleClearance")) return false;
+    clearance_radius = (radius == 0 && margin == 0) ? 0.0 : radius;
+    return true;
+}
+
+// The obstacle-goal rule extended to the lethal ring of the obstacle clearance: the rover cannot stand
+// on a goal whose clearance is <= radius, so it is refused like a goal on an obstacle.
+bool DyMuPathPlanner::goalInLethalRing()
+{
+    if (!(clearance_radius > 0)) return false;
+    uint32_t idx = goal_j * num_nodes_X + goal_i;
+    double d = kInf;
+    if (!deviceOk(dymu_read_cells(dev, DYMU_PLANE_CLEARANCE, 0, &idx, 1, &d), "goal clearance")) return true;
+    return d <= clearance_radius;
 }
 
 void DyMuPathPlanner::finishReadback()
@@ -370,7 +392,7 @@ bool DyMuPathPlanner::computeTotalCostMap(base::Waypoint wPos)
         return false;
     }
     readNode(goal_i, goal_j, goal_view);
-    if (goal_view.isObstacle)
+    if (goal_view.isObstacle || goalInLethalRing())
     {
         LOG_WARN_S << "The goal is not valid";
         return false;
@@ -467,6 +489,11 @@ bool DyMuPathPlanner::computeEntireTotalCostMap()
             LOG_WARN_S << "The goal is not valid";
             return false;
         }
+    }
+    if (goalInLethalRing())
+    {
+        LOG_WARN_S << "The goal is not valid";
+        return false;
     }
     // With a cost map that is still being uploaded (setCostMap(const double*, ld)) the test
     // "global_goal->isObstacle" (G.cpp:447) is left to the solve itself, which starts on the rows
