@@ -335,6 +335,55 @@ int dymu_batch_solve(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_goals, const ui
                      const uint32_t* goal_j, const double* start_xy, double tau, double* paths,
                      uint32_t cap, uint32_t* path_len, int32_t* path_status, float* ms_per_ctx);
 
+/* ---- batches of independent cost maps (an extension; the reference holds one map) -------------
+ * Map q of a batch is solved into total-cost slot q and has its own cost-term plane C_eff_q.  A map is
+ * given as its cost matrix (ny x nx, row stride ld) and is self-contained: C_eff_q equals, bit for bit,
+ * the DYMU_PLANE_CEFF that a freshly created context of the same size and resolutions builds from
+ * dymu_set_cost_map(cost_q) (setCostMap, G.cpp:109-126, with hazard_density 0 and trafficability 1):
+ *     +inf                                  where cost <= 0 (obstacle)
+ *     global_res * cost * (2 + 0.0 - 1.0)   otherwise
+ * The context's own hazard_density, trafficability, obstacles, clearance and anisotropy are not
+ * applied.  A cost that is neither <= 0 nor gives a finite C_eff (NaN, +inf, overflow) is DYMU_ERR_ARG
+ * and leaves that map unset.  A goal on a cell with C_eff_q = +inf is not seeded (counted in
+ * stats.goal_obstacle) and slot q stays +inf.  The tile solver's priority band of a launch is
+ * kBandFactor * tile * the mean of the finite C_eff of all its maps.
+ * Results are read with the slot-based calls: dymu_download_total_cost, dymu_read_cells,
+ * dymu_count_reached, dymu_stop_threshold, dymu_extract_global_path[_batch] (waypoint z from the
+ * context's elevation plane).  On the device, slot q lives at
+ * dymu_plane_device_ptr(DYMU_PLANE_TOTAL_COST) + q * pitch * rows (dymu_geometry).
+ * A map solve overwrites slots [0, n): the context's resident solve is gone (the next
+ * dymu_solve_incremental is a full solve) and direct delivery (dymu_set_total_cost_export) is never
+ * used, even for n == 1.  The context's cost, obstacle, C_eff and export planes are not touched.
+ * With slope anisotropy or obstacle clearance on, dymu_solve_maps and dymu_batch_solve_maps return
+ * DYMU_ERR_STATE. */
+/* n C_eff planes (map q <-> total-cost slot q); grows the slots to n if fewer; n = 0 frees them.  A
+ * different count drops every map set before. */
+int dymu_reserve_maps(dymu_ctx* ctx, uint32_t n_maps);
+/* maps [first, first+n) from n dense matrices of the context's ny rows and nx columns, row stride ld,
+   matrix stride map_stride (doubles); device_ptr != 0: device memory of this GPU (the caller has
+   finished writing it), the whole range from cost to the last cell of the last matrix inside one
+   allocation (only its first and last cells are checked); returns when the maps are in the context.
+   first + n above the reserved maps is DYMU_ERR_ARG. */
+int dymu_set_maps(dymu_ctx* ctx, uint32_t first, uint32_t n, const double* cost, size_t ld,
+                  size_t map_stride, int device_ptr);
+/* computeEntireTotalCostMap (G.cpp:443-468) of map q toward goal q into slot q, q < n, one launch.
+ * n above the reserved maps or the slots is DYMU_ERR_ARG, a map never set DYMU_ERR_STATE.  `stats`
+ * may be NULL or point to one entry (aggregate over the launch). */
+int dymu_solve_maps(dymu_ctx* ctx, uint32_t n, const uint32_t* goal_i, const uint32_t* goal_j,
+                    dymu_solve_stats* stats);
+/* dymu_batch_solve for maps: context k gets the k-th contiguous block, one host thread per context,
+   in chunks of its reserved maps (every context needs dymu_reserve_maps >= 1 and the size of the
+   others); map q is costs + q*map_stride (host memory, ny rows of row stride ld, ny and nx those of
+   the contexts: the caller's buffers must hold n_maps such matrices).  Optional paths (format of
+   dymu_extract_global_path: paths + q*cap*5, path_len[q], path_status[q], from start_xy[2q..2q+1])
+   and optional total-cost matrices (n_maps x ny x tc_ld, XFORM_NONE).  ms_per_ctx (optional): host
+   wall time of each context's share. */
+int dymu_batch_solve_maps(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_maps, const double* costs,
+                          size_t ld, size_t map_stride, const uint32_t* goal_i, const uint32_t* goal_j,
+                          const double* start_xy, double tau, double* paths, uint32_t cap,
+                          uint32_t* path_len, int32_t* path_status, double* total_cost, size_t tc_ld,
+                          float* ms_per_ctx);
+
 typedef struct dymu_dd_stats
 {
     uint32_t rounds;            /* exchange rounds */

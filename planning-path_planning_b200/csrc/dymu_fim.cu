@@ -46,7 +46,9 @@
 // (see Params::tmax); k_deliver_rest stores what is left.  A waiting CTA gives up after eight
 // seconds at the grid barrier (barrier_spin) and the solve returns an error instead of hanging.
 // The same kernel runs the local layer's risk dilation (propagateRisk,
-// src/DyMu_LocalPathRepairing.cpp:550-576) in MODE 1, a max-propagation on risk.
+// src/DyMu_LocalPathRepairing.cpp:550-576) in MODE 1, a max-propagation on risk, and a batch of
+// independent maps (dymu_solve_maps) in MODE 3: MODE 0 with problem q reading its own cost-term
+// plane at C + q * slot_stride.
 #include <cooperative_groups.h>
 #include <stdlib.h>
 
@@ -239,7 +241,7 @@ template <int MODE>
 __device__ __forceinline__ bool relax(double tc, double tl, double tr, double tu, double td,
                                       double c, double cc2 /* 2 c^2 */, double& out)
 {
-    if (MODE == 0)
+    if (MODE != 1)  // MODE 0 / 3
     {
         // No guards around the square root: the argument 2c^2 - d^2 lies in [c^2, 2c^2] whenever
         // the two-sided value is selected; otherwise (one side +inf, both +inf -> d NaN, or a
@@ -493,7 +495,8 @@ __global__ void __launch_bounds__(THREADS, MIN_CTAS) k_fim(Params p)
             const uint32_t why = ld_volatile_u32(&flag_cur[tile_id]);
             double* Tg = p.T + (size_t)prob * p.slot_stride + (size_t)ty * TILE * p.pitch
                          + (size_t)tx * TILE;
-            const double* Cg = p.C + (size_t)ty * TILE * p.pitch + (size_t)tx * TILE;
+            const double* Cg = p.C + (MODE == 3 ? (size_t)prob * p.slot_stride : 0)
+                               + (size_t)ty * TILE * p.pitch + (size_t)tx * TILE;
 
             // ---- stage the tile: T interior + halo (L2-coherent loads: other CTAs write
             // T during this phase), C through the read-only path
@@ -890,6 +893,32 @@ __global__ void k_seed(double* T, size_t slot_stride, uint32_t pitch, uint32_t n
     if (n_seeded) gmin[0] = 0ull;
 }
 
+// k_seed for a map batch: goal q is tested against its own cost-term plane (C_eff = +inf: obstacle)
+__global__ void k_seed_maps(double* T, size_t slot_stride, uint32_t pitch, uint32_t ntx, uint32_t nty,
+                            const uint32_t* goal_ij, uint32_t n, const double* ceff, uint32_t* list0,
+                            uint32_t* flag0, unsigned long long* key0, unsigned long long* gmin,
+                            uint32_t* ctrl, unsigned long long* stats)
+{
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    uint32_t n_seeded = 0;
+    for (uint32_t q = 0; q < n; ++q)
+    {
+        const size_t cell = (size_t)goal_ij[2 * q + 1] * pitch + goal_ij[2 * q];
+        if (!(ceff[(size_t)q * slot_stride + cell] < DYMU_INF))
+        {
+            stats[kStatGoalObstacle]++;
+            continue;
+        }
+        T[(size_t)q * slot_stride + cell] = 0.0;
+        const uint32_t tile_id = q * ntx * nty + (goal_ij[2 * q + 1] / TILE) * ntx + goal_ij[2 * q] / TILE;
+        flag0[tile_id] = kFull;
+        key0[tile_id] = 0ull;
+        list0[n_seeded++] = tile_id;
+    }
+    ctrl[kCtrlCount] = n_seeded;
+    if (n_seeded) gmin[0] = 0ull;
+}
+
 __global__ void k_seed_all(uint32_t n, uint32_t* list0, uint32_t* flag0, unsigned long long* key0,
                            unsigned long long* gmin, uint32_t* ctrl)
 {
@@ -1069,6 +1098,17 @@ int dymu_internal_fim_clear(dymu_ctx* ctx, dymu_fim_work* w)
     return DYMU_OK;
 }
 
+int dymu_internal_fim_seed_maps(dymu_ctx* ctx, dymu_fim_work* w, const uint32_t* d_goal_ij, uint32_t n)
+{
+    DYMU_TRY(dymu_internal_fim_clear(ctx, w));
+    k_seed_maps<<<1, 32, 0, ctx->stream>>>(ctx->T, (size_t)ctx->pitch * ctx->rows, ctx->pitch, ctx->ntx, ctx->nty,
+                                           d_goal_ij, n, ctx->maps, w->list[0], w->flag[0], w->key[0], w->gmin,
+                                           w->ctrl, w->stats);
+    ctx->launches++;
+    DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    return DYMU_OK;
+}
+
 int dymu_internal_fim_seed_all(dymu_ctx* ctx, dymu_fim_work* w, uint32_t n_tiles)
 {
     DYMU_TRY(dymu_internal_fim_clear(ctx, w));
@@ -1159,7 +1199,8 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
     if (L.mode == 2 && !L.A) DYMU_FAIL(ctx, DYMU_ERR_STATE, "anisotropic solve without directional costs");
     rc = (L.mode == 0)   ? launch_fim<0>(ctx, prm, total_tiles)
          : (L.mode == 1) ? launch_fim<1>(ctx, prm, total_tiles)
-                         : launch_fim<2>(ctx, prm, total_tiles);
+         : (L.mode == 2) ? launch_fim<2>(ctx, prm, total_tiles)
+                         : launch_fim<3>(ctx, prm, total_tiles);
     DYMU_TRY(rc);
     DYMU_CUDA_TRY(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
     if (prm.xout)

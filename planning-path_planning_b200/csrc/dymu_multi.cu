@@ -5,6 +5,8 @@
 //                     out in contiguous blocks, one host thread per context, no data-path
 //                     exchange at all (the reference would run one planner instance per query:
 //                     computeEntireTotalCostMap G.cpp:443-468 + getPath G.cpp:589-611).
+//                     dymu_batch_solve_maps deals out (map, goal) pairs the same way, each
+//                     context taking its block in chunks of its reserved maps (dymu_maps.cu).
 //   dymu_dd_solve     ONE grid cut into row strips, one strip per context.  A strip carries one
 //                     ghost row per interior side whose cost is 0 (obstacle: never a propagation
 //                     target), so it acts as Dirichlet data.  Every round each strip advances by
@@ -175,6 +177,12 @@ struct BatchShared
     dymu_ctx** ctxs;
     uint32_t n_ctx, n_goals;
     const uint32_t *goal_i, *goal_j;
+    // map batches: query q solves the cost map at costs + q * map_stride (nullptr: every query on the
+    // context's own map) and, if total_cost is given, stores its matrix at total_cost + q * ny * tc_ld
+    const double* costs;
+    size_t ld, map_stride;
+    double* total_cost;
+    size_t tc_ld;
     const double* start_xy;
     double tau;
     double* paths;
@@ -201,7 +209,7 @@ void* batch_worker(void* arg)
     // contiguous block of queries (sizes differ by at most one)
     const uint32_t base = S.n_goals / S.n_ctx, extra = S.n_goals % S.n_ctx;
     const uint32_t lo = k * base + (k < extra ? k : extra), cnt = base + (k < extra ? 1u : 0u);
-    const uint32_t B = ctx->n_slots;
+    const uint32_t B = S.costs ? ctx->n_maps : ctx->n_slots;
     std::vector<uint32_t> slots(B), gij(2 * (size_t)B);
     int rc = DYMU_OK;
     const double t0 = now_ms();
@@ -209,7 +217,16 @@ void* batch_worker(void* arg)
     {
         const uint32_t m = (cnt - q0 < B) ? cnt - q0 : B;
         dymu_solve_stats st;
-        rc = dymu_solve_total_cost(ctx, m, S.goal_i + lo + q0, S.goal_j + lo + q0, &st);
+        if (S.costs)
+        {
+            rc = dymu_set_maps(ctx, 0, m, S.costs + (size_t)(lo + q0) * S.map_stride, S.ld, S.map_stride, 0);
+            if (rc == DYMU_OK) rc = dymu_solve_maps(ctx, m, S.goal_i + lo + q0, S.goal_j + lo + q0, &st);
+            for (uint32_t s = 0; s < m && rc == DYMU_OK && S.total_cost; ++s)
+                rc = dymu_download_total_cost(ctx, s, S.total_cost + (size_t)(lo + q0 + s) * ctx->ny * S.tc_ld,
+                                              S.tc_ld, DYMU_XFORM_NONE);
+        }
+        else
+            rc = dymu_solve_total_cost(ctx, m, S.goal_i + lo + q0, S.goal_j + lo + q0, &st);
         if (rc != DYMU_OK || !S.start_xy || !S.paths) continue;
         for (uint32_t s = 0; s < m; ++s)
         {
@@ -225,6 +242,29 @@ void* batch_worker(void* arg)
     S.ms[k] = (float)(now_ms() - t0);
     S.rc[k] = rc;
     return nullptr;
+}
+
+// one batch_worker thread per context; the first failure is returned
+int run_batch(BatchShared& S, float* ms_per_ctx)
+{
+    S.rc.assign(S.n_ctx, DYMU_OK);
+    S.ms.assign(S.n_ctx, 0.f);
+    std::vector<pthread_t> th(S.n_ctx);
+    std::vector<BatchThread> args(S.n_ctx);
+    for (uint32_t k = 0; k < S.n_ctx; ++k)
+    {
+        args[k].s = &S;
+        args[k].k = k;
+        pthread_create(&th[k], nullptr, batch_worker, &args[k]);
+    }
+    int rc = DYMU_OK;
+    for (uint32_t k = 0; k < S.n_ctx; ++k)
+    {
+        pthread_join(th[k], nullptr);
+        if (S.rc[k] != DYMU_OK && rc == DYMU_OK) rc = S.rc[k];
+        if (ms_per_ctx) ms_per_ctx[k] = S.ms[k];
+    }
+    return rc;
 }
 }  // namespace
 
@@ -340,24 +380,35 @@ int dymu_batch_solve(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_goals, const ui
     S.ctxs = ctxs; S.n_ctx = n_ctx; S.n_goals = n_goals; S.goal_i = goal_i; S.goal_j = goal_j;
     S.start_xy = start_xy; S.tau = tau; S.paths = paths; S.cap = cap; S.path_len = path_len;
     S.path_status = path_status;
-    S.rc.assign(n_ctx, DYMU_OK);
-    S.ms.assign(n_ctx, 0.f);
-    std::vector<pthread_t> th(n_ctx);
-    std::vector<BatchThread> args(n_ctx);
+    S.costs = nullptr; S.ld = S.map_stride = S.tc_ld = 0; S.total_cost = nullptr;
+    return run_batch(S, ms_per_ctx);
+}
+
+int dymu_batch_solve_maps(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_maps, const double* costs,
+                          size_t ld, size_t map_stride, const uint32_t* goal_i, const uint32_t* goal_j,
+                          const double* start_xy, double tau, double* paths, uint32_t cap,
+                          uint32_t* path_len, int32_t* path_status, double* total_cost, size_t tc_ld,
+                          float* ms_per_ctx)
+{
+    if (!ctxs || n_ctx < 1 || !costs || !goal_i || !goal_j) return DYMU_ERR_ARG;
+    if (paths && (!start_xy || !path_len || !path_status || cap == 0)) return DYMU_ERR_ARG;
     for (uint32_t k = 0; k < n_ctx; ++k)
     {
-        args[k].s = &S;
-        args[k].k = k;
-        pthread_create(&th[k], nullptr, batch_worker, &args[k]);
+        dymu_ctx* c = ctxs[k];
+        if (!c) return DYMU_ERR_ARG;
+        if (c->nx != ctxs[0]->nx || c->ny != ctxs[0]->ny || ld < c->nx || (total_cost && tc_ld < c->nx))
+            DYMU_FAIL(c, DYMU_ERR_ARG, "context %u: every context has the size of the maps (ld, tc_ld >= nx)", k);
+        if (c->n_maps == 0) DYMU_FAIL(c, DYMU_ERR_STATE, "context %u has no reserved maps (dymu_reserve_maps)", k);
+        if (c->aniso_n || c->clear_on)
+            DYMU_FAIL(c, DYMU_ERR_STATE, "context %u: map batches are isotropic and without obstacle clearance", k);
     }
-    int rc = DYMU_OK;
-    for (uint32_t k = 0; k < n_ctx; ++k)
-    {
-        pthread_join(th[k], nullptr);
-        if (S.rc[k] != DYMU_OK && rc == DYMU_OK) rc = S.rc[k];
-        if (ms_per_ctx) ms_per_ctx[k] = S.ms[k];
-    }
-    return rc;
+    if (n_maps == 0) return DYMU_OK;
+    BatchShared S;
+    S.ctxs = ctxs; S.n_ctx = n_ctx; S.n_goals = n_maps; S.goal_i = goal_i; S.goal_j = goal_j;
+    S.start_xy = start_xy; S.tau = tau; S.paths = paths; S.cap = cap; S.path_len = path_len;
+    S.path_status = path_status;
+    S.costs = costs; S.ld = ld; S.map_stride = map_stride; S.total_cost = total_cost; S.tc_ld = tc_ld;
+    return run_batch(S, ms_per_ctx);
 }
 
 }  // extern "C"

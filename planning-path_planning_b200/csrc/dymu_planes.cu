@@ -10,9 +10,6 @@
 namespace
 {
 constexpr int kThreads = 256;
-// band width of the tile scheduler (dymu_fim.cu) in units of tile * mean(C_eff): a few tile
-// crossings worth of total cost (DESIGN.md section 5: flat around 4 over a grid of 24 settings)
-constexpr double kBandFactor = 4.0;
 
 inline int stream_grid(const dymu_ctx* ctx, size_t work_items, int per_thread = 1)
 {
@@ -566,6 +563,7 @@ int dymu_destroy(dymu_ctx* ctx)
     dymu_internal_local_free(ctx);
     dymu_internal_incremental_free(ctx);
     dymu_internal_clearance_free(ctx);
+    dymu_internal_maps_free(ctx);
     dymu_internal_fim_free(&ctx->work);
     void* ptrs[] = {ctx->elev, ctx->slope, ctx->raw, ctx->cost, ctx->haz, ctx->traff, ctx->ceff,
                     ctx->T, ctx->terrain, ctx->obst, ctx->locmode, ctx->d_lut, ctx->d_slopes,

@@ -77,6 +77,12 @@ _SIG = {
                                 C.POINTER(DdStats)]),
     "dymu_batch_solve": (C.c_int, [C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, _u32p, _u32p, _dp, C.c_double,
                                    _dp, C.c_uint32, _u32p, C.POINTER(C.c_int32), C.POINTER(C.c_float)]),
+    "dymu_reserve_maps": (C.c_int, [C.c_void_p, C.c_uint32]),
+    "dymu_set_maps": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_size_t, C.c_size_t, C.c_int]),
+    "dymu_solve_maps": (C.c_int, [C.c_void_p, C.c_uint32, _u32p, _u32p, C.POINTER(SolveStats)]),
+    "dymu_batch_solve_maps": (C.c_int, [C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, _dp, C.c_size_t, C.c_size_t,
+                                        _u32p, _u32p, _dp, C.c_double, _dp, C.c_uint32, _u32p,
+                                        C.POINTER(C.c_int32), _dp, C.c_size_t, C.POINTER(C.c_float)]),
     "dymu_local_reshape": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int64, C.c_int64]),
     "dymu_solve_incremental": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(SolveStats),
                                          C.POINTER(C.c_uint64)]),
@@ -310,6 +316,34 @@ class DeviceLayer:
         st = SolveStats()
         self._chk(self._l.dymu_solve_total_cost(self._h, g.shape[0], gi.ctypes.data_as(_u32p),
                                                 gj.ctypes.data_as(_u32p), C.byref(st)))
+        return st.as_dict()
+
+    # map batches (map q <-> total-cost slot q; read the slots with the slot-based calls)
+    def reserve_maps(self, n):
+        """n cost-term planes, one per total-cost slot (grows the slots to n); 0 frees them."""
+        self._chk(self._l.dymu_reserve_maps(self._h, int(n)))
+
+    def set_maps(self, costs, first=0):
+        """Maps [first, first+n) from a numpy (n, ny, nx) (or (ny, nx)) array of costs."""
+        a = _f64(costs)
+        a = a.reshape((-1,) + a.shape[-2:])
+        if a.shape[1:] != (self.ny, self.nx):
+            raise ValueError("expected maps of shape (%d, %d)" % (self.ny, self.nx))
+        self._chk(self._l.dymu_set_maps(self._h, int(first), a.shape[0], C.c_void_p(a.ctypes.data),
+                                        a.shape[2], a.shape[1] * a.shape[2], 0))
+
+    def set_maps_device(self, ptr, n, ld, map_stride, first=0):
+        """Maps [first, first+n) from device memory of this GPU (e.g. a torch CUDA tensor's data_ptr(),
+        after the stream that wrote it was synchronised); ld, map_stride in doubles."""
+        self._chk(self._l.dymu_set_maps(self._h, int(first), int(n), C.c_void_p(ptr), int(ld), int(map_stride), 1))
+
+    def solve_maps(self, goals):
+        """goals[q] = (i, j) of map q, solved into slot q in one launch.  Returns the aggregate SolveStats."""
+        g = np.asarray(list(goals), dtype=np.uint32).reshape(-1, 2)
+        gi, gj = np.ascontiguousarray(g[:, 0]), np.ascontiguousarray(g[:, 1])
+        st = SolveStats()
+        self._chk(self._l.dymu_solve_maps(self._h, g.shape[0], gi.ctypes.data_as(_u32p), gj.ctypes.data_as(_u32p),
+                                          C.byref(st)))
         return st.as_dict()
 
     def solve_incremental(self, goal):
@@ -587,3 +621,45 @@ def batch_solve(layers, goals, starts=None, tau=0.4, cap=1 << 14):
         texts = [lib.dymu_last_error(d._h).decode() for d in layers]
         raise DymuError(rc, "; ".join(t for t in texts if t))
     return paths, ms
+
+
+def batch_solve_maps(layers, costs, goals, starts=None, tau=0.4, cap=1 << 14, total_cost=False):
+    """dymu_batch_solve_maps: map q of `costs` (numpy (n, ny, nx)) toward goals[q], dealt out over
+    `layers` (same size, reserve_maps() maps per launch each).  Returns (paths or None, total-cost
+    matrices (n, ny, nx) or None, per-context wall ms)."""
+    lib = load_library()
+    a = _f64(costs)
+    if a.ndim != 3:
+        raise ValueError("costs must be an (n, ny, nx) array of maps")
+    n, ny, nx = a.shape
+    # the library reads and writes ny rows of nx cells per map, with ny and nx taken from the contexts
+    for d in layers:
+        if (d.ny, d.nx) != (ny, nx):
+            raise ValueError("maps of shape (%d, %d) for a layer of shape (%d, %d)" % (ny, nx, d.ny, d.nx))
+    g = np.ascontiguousarray(goals, dtype=np.uint32).reshape(-1, 2)
+    if g.shape[0] != n:
+        raise ValueError("one goal per map")
+    gi, gj = np.ascontiguousarray(g[:, 0]), np.ascontiguousarray(g[:, 1])
+    ms = np.zeros(len(layers), dtype=np.float32)
+    xy = out = ln = stt = None
+    if starts is not None:
+        xy = np.ascontiguousarray(starts, dtype=np.float64)
+        if xy.size != 2 * n:
+            raise ValueError("one start (x, y) per map")
+        xy = xy.reshape(n, 2)
+        out = np.empty((n, cap, 5), dtype=np.float64)
+        ln = np.zeros(n, dtype=np.uint32)
+        stt = np.zeros(n, dtype=np.int32)
+    T = np.empty((n, ny, nx), dtype=np.float64) if total_cost else None
+    rc = lib.dymu_batch_solve_maps(
+        _ctx_array(layers), len(layers), n, a.ctypes.data_as(_dp), nx, ny * nx, gi.ctypes.data_as(_u32p),
+        gj.ctypes.data_as(_u32p), xy.ctypes.data_as(_dp) if xy is not None else None, float(tau),
+        out.ctypes.data_as(_dp) if out is not None else None, int(cap) if out is not None else 0,
+        ln.ctypes.data_as(_u32p) if ln is not None else None,
+        stt.ctypes.data_as(C.POINTER(C.c_int32)) if stt is not None else None,
+        T.ctypes.data_as(_dp) if T is not None else None, nx, ms.ctypes.data_as(C.POINTER(C.c_float)))
+    if rc != 0:
+        texts = [lib.dymu_last_error(d._h).decode() for d in layers]
+        raise DymuError(rc, "; ".join(t for t in texts if t))
+    paths = [(out[q, :ln[q]].copy(), int(stt[q])) for q in range(n)] if out is not None else None
+    return paths, T, ms
