@@ -354,8 +354,23 @@ int dymu_batch_solve(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_goals, const ui
  * A map solve overwrites slots [0, n): the context's resident solve is gone (the next
  * dymu_solve_incremental is a full solve) and direct delivery (dymu_set_total_cost_export) is never
  * used, even for n == 1.  The context's cost, obstacle, C_eff and export planes are not touched.
- * With slope anisotropy or obstacle clearance on, dymu_solve_maps and dymu_batch_solve_maps return
- * DYMU_ERR_STATE. */
+ * With the context's own slope anisotropy or obstacle clearance on, dymu_solve_maps and
+ * dymu_batch_solve_maps return DYMU_ERR_STATE: map batches have settings of their own
+ * (dymu_set_maps_clearance, dymu_set_maps_anisotropy, both off by default, applied at solve time).  With
+ * them, map q solved toward goal g_q equals a freshly created context of the same size and resolutions
+ * that was given the batch context's DYMU_PLANE_ELEVATION, then dymu_set_cost_map(cost_q),
+ * dymu_set_obstacle_clearance and dymu_set_anisotropy with the batch parameters, and solved with
+ * dymu_solve_total_cost({g_q}): its C_eff, directional costs and clearance bit for bit, its total cost to
+ * rounding.  Goals are seeded as there: one on an obstacle (cost <= 0) is not seeded, one inside the
+ * lethal ring is.  The priority band of an anisotropic launch is kBandFactor * tile * the mean of the
+ * finite directional costs of all its maps.  The descent (dymu_extract_global_path[_batch]) on a slot
+ * written by an anisotropic map solve follows that solve's metric; after the map was set again, a batch
+ * setting changed, the maps were reserved again, or a later anisotropic map solve over fewer maps rebuilt
+ * the factor planes from the elevation, it is DYMU_ERR_STATE on that slot until something writes the
+ * slot again.  Every other writer of a slot (dymu_solve_total_cost and the other context solves,
+ * dymu_reset_total_cost, dymu_import_rows_min_key, dymu_reserve_slots, an isotropic map solve) gives it
+ * the context's own descent again.  Memory: batch clearance adds one fp64 and one u8 plane per reserved
+ * map, batch anisotropy four fp64 planes per context. */
 /* n C_eff planes (map q <-> total-cost slot q); grows the slots to n if fewer; n = 0 frees them.  A
  * different count drops every map set before. */
 int dymu_reserve_maps(dymu_ctx* ctx, uint32_t n_maps);
@@ -383,6 +398,17 @@ int dymu_batch_solve_maps(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_maps, cons
                           const double* start_xy, double tau, double* paths, uint32_t cap,
                           uint32_t* path_len, int32_t* path_status, double* total_cost, size_t tc_ld,
                           float* ms_per_ctx);
+/* Each context of dymu_batch_solve_maps solves with its own batch settings; contexts whose batch
+   clearance parameters or anisotropy tables differ are DYMU_ERR_ARG before any work.  With batch
+   anisotropy on, each context's DYMU_PLANE_ELEVATION is the caller's to set, the same on all of them. */
+/* obstacle clearance of every map solve of this context: same parameters, validation and off switch
+   (radius == 0 && margin == 0) as dymu_set_obstacle_clearance.  The obstacles of map q are its cells with
+   cost <= 0.  The adjusted planes are built at the next dymu_solve_maps, for the maps that changed. */
+int dymu_set_maps_clearance(dymu_ctx* ctx, double radius, double margin, double penalty);
+/* slope anisotropy of every map solve: same table rules and off switch (n == 0) as dymu_set_anisotropy;
+   the elevation is the context's DYMU_PLANE_ELEVATION as it is at each dymu_solve_maps, shared by all
+   maps */
+int dymu_set_maps_anisotropy(dymu_ctx* ctx, const double* theta_deg, const double* factor, int n);
 
 typedef struct dymu_dd_stats
 {

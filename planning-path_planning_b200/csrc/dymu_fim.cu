@@ -48,7 +48,8 @@
 // The same kernel runs the local layer's risk dilation (propagateRisk,
 // src/DyMu_LocalPathRepairing.cpp:550-576) in MODE 1, a max-propagation on risk, and a batch of
 // independent maps (dymu_solve_maps) in MODE 3: MODE 0 with problem q reading its own cost-term
-// plane at C + q * slot_stride.
+// plane at C + q * slot_stride.  MODE 4 is the anisotropic map batch: MODE 2 with the directional
+// costs staged as C_q(x) * A_d(x), C_q read as in MODE 3 and A the four factor planes f(theta(x->m)).
 #include <cooperative_groups.h>
 #include <stdlib.h>
 
@@ -72,7 +73,7 @@ constexpr int CPT = TILE * TILE / THREADS;  // cells per thread in load/store = 
 constexpr int MIN_CTAS = 2;  // 1024 threads per SM: caps a thread at 64 registers
 constexpr int SWEEP_CAP = 2 * TILE;  // sweeps per activation; the rest resumes next phase
 constexpr size_t SMEM = sizeof(double) * ((TILE + 2) * PITCH + TILE * PITCH);
-// MODE 2 stages the four directional costs of the tile instead of one cost term
+// MODE 2 / 4 stage the four directional costs of the tile instead of one cost term
 constexpr size_t SMEM_ANISO = sizeof(double) * ((TILE + 2) * PITCH + 4 * TILE * PITCH);
 
 // activation flag bits: which halo of the tile is stale / whole tile must be re-evaluated
@@ -114,7 +115,8 @@ struct Params
     int xminus1;                // +inf is delivered as -1 (getTotalCostMatrix, G.cpp:799-811)
     const uint32_t* stop_flag;  // leave after the phase in which *stop_flag >= stop_value (nullptr: never)
     uint32_t stop_value;
-    // MODE 2: the directional costs a(x->m), four planes in the order i-1, i+1, j-1, j+1
+    // MODE 2: the directional costs a(x->m), four planes in the order i-1, i+1, j-1, j+1;
+    // MODE 4: the factors f(theta(x->m)) in the same order, shared by all problems
     const double* A;
     size_t a_stride;            // doubles between two of those planes
 };
@@ -495,7 +497,7 @@ __global__ void __launch_bounds__(THREADS, MIN_CTAS) k_fim(Params p)
             const uint32_t why = ld_volatile_u32(&flag_cur[tile_id]);
             double* Tg = p.T + (size_t)prob * p.slot_stride + (size_t)ty * TILE * p.pitch
                          + (size_t)tx * TILE;
-            const double* Cg = p.C + (MODE == 3 ? (size_t)prob * p.slot_stride : 0)
+            const double* Cg = p.C + (MODE == 3 || MODE == 4 ? (size_t)prob * p.slot_stride : 0)
                                + (size_t)ty * TILE * p.pitch + (size_t)tx * TILE;
 
             // ---- stage the tile: T interior + halo (L2-coherent loads: other CTAs write
@@ -546,6 +548,16 @@ __global__ void __launch_bounds__(THREADS, MIN_CTAS) k_fim(Params p)
                     for (int q = 0; q < 4; ++q)
                         Cs[q * TILE * P + y * P + x] =
                             __ldg(&p.A[q * p.a_stride + (size_t)(ty * TILE + y) * p.pitch + tx * TILE + x]);
+                }
+                else if constexpr (MODE == 4)
+                {
+                    // k_dircost's a(x->m) = C_eff(x) * f, bit for bit: +inf for an impassable cell (C_q
+                    // = +inf) and toward an outside neighbour (f = +inf), overflow included
+                    const double c = __ldg(&Cg[(size_t)y * p.pitch + x]);
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        Cs[q * TILE * P + y * P + x] =
+                            c * __ldg(&p.A[q * p.a_stride + (size_t)(ty * TILE + y) * p.pitch + tx * TILE + x]);
                 }
                 else
                     Cs[y * P + x] = __ldg(&Cg[(size_t)y * p.pitch + x]);
@@ -608,7 +620,7 @@ __global__ void __launch_bounds__(THREADS, MIN_CTAS) k_fim(Params p)
                         asm volatile("" : "+d"(tA));
                         double nA, nB;
                         bool chA;
-                        if constexpr (MODE == 2)
+                        if constexpr (MODE == 2 || MODE == 4)
                             chA = relax_aniso(tA, lA, rA, uA, dA, a + c_off, TILE * P, nA);
                         else
                             chA = relax<MODE>(tA, lA, rA, uA, dA, cA, qA, nA);
@@ -618,7 +630,7 @@ __global__ void __launch_bounds__(THREADS, MIN_CTAS) k_fim(Params p)
                         const double tB = b[0];
                         const double lB = b[-1], rB = b[1], uB = b[-P], dB = b[P];
                         bool chB;
-                        if constexpr (MODE == 2)
+                        if constexpr (MODE == 2 || MODE == 4)
                             chB = relax_aniso(tB, lB, rB, uB, dB, b + c_off, TILE * P, nB);
                         else
                             chB = relax<MODE>(tB, lB, rB, uB, dB, cB, qB, nB);
@@ -999,7 +1011,7 @@ __global__ void k_import_rows_min(double* T, uint32_t pitch, uint32_t nx, uint32
 
 template <int MODE> int launch_fim(dymu_ctx* ctx, Params& prm, size_t total_tiles)
 {
-    constexpr size_t smem = MODE == 2 ? SMEM_ANISO : SMEM;
+    constexpr size_t smem = (MODE == 2 || MODE == 4) ? SMEM_ANISO : SMEM;
     // persistent grid = every CTA that can be co-resident (required by the grid barrier)
     int per_sm = 0;
     DYMU_CUDA_TRY(ctx, cudaFuncSetAttribute(k_fim<MODE>,
@@ -1196,11 +1208,13 @@ int dymu_internal_fim_run(dymu_ctx* ctx, const dymu_fim_launch& L, dymu_solve_st
     w->unclean = true;  // until this launch reports that it drained its lists
     DYMU_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     int rc;
-    if (L.mode == 2 && !L.A) DYMU_FAIL(ctx, DYMU_ERR_STATE, "anisotropic solve without directional costs");
+    if ((L.mode == 2 || L.mode == 4) && !L.A)
+        DYMU_FAIL(ctx, DYMU_ERR_STATE, "anisotropic solve without directional costs");
     rc = (L.mode == 0)   ? launch_fim<0>(ctx, prm, total_tiles)
          : (L.mode == 1) ? launch_fim<1>(ctx, prm, total_tiles)
          : (L.mode == 2) ? launch_fim<2>(ctx, prm, total_tiles)
-                         : launch_fim<3>(ctx, prm, total_tiles);
+         : (L.mode == 3) ? launch_fim<3>(ctx, prm, total_tiles)
+                         : launch_fim<4>(ctx, prm, total_tiles);
     DYMU_TRY(rc);
     DYMU_CUDA_TRY(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
     if (prm.xout)
@@ -1340,6 +1354,7 @@ int dymu_reserve_slots(dymu_ctx* ctx, uint32_t n_slots)
     ctx->n_slots = n_slots;
     DYMU_TRY(dymu_internal_fill(ctx, ctx->T, 1.0 / 0.0, n * n_slots));
     DYMU_TRY(dymu_internal_fim_alloc(ctx, &ctx->work, (size_t)ctx->ntx * ctx->nty * n_slots));
+    dymu_internal_unmark_all(ctx);
     ctx->solved = false;
     return DYMU_OK;
 }
@@ -1358,6 +1373,7 @@ static int solve_total_cost_impl(dymu_ctx* ctx, uint32_t n_goals, const uint32_t
     // resetTotalCostMap, G.cpp:473-485 (whole plane instead of the propagated-node list)
     DYMU_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     DYMU_TRY(dymu_internal_fill(ctx, ctx->T, 1.0 / 0.0, n * n_goals));
+    dymu_internal_unmark_slots(ctx, 0, n_goals);
     DYMU_TRY(dymu_internal_scratch(ctx, (size_t)n_goals * 8, (size_t)n_goals * 8));
     uint32_t* h_goals = (uint32_t*)ctx->h_pinned;
     for (uint32_t q = 0; q < n_goals; ++q)
@@ -1462,6 +1478,7 @@ static int solve_resume_impl(dymu_ctx* ctx, const uint32_t* ranges, uint32_t n_r
         if (ranges[2 * k] >= ranges[2 * k + 1] || ranges[2 * k + 1] > ctx->ny) return DYMU_ERR_ARG;
     DYMU_TRY(dymu_internal_refresh_ceff(ctx));
     DYMU_TRY(dymu_internal_settle_delivery(ctx));
+    dymu_internal_unmark_slots(ctx, 0, 1);
     // distinct tile rows covered by the ranges
     DYMU_TRY(dymu_internal_scratch(ctx, sizeof(uint32_t) * ctx->nty, sizeof(uint32_t) * ctx->nty));
     uint32_t* h_rows = (uint32_t*)ctx->h_pinned;
@@ -1716,6 +1733,7 @@ int dymu_reset_total_cost(dymu_ctx* ctx)
     ctx->solved = false;
     ctx->export_done = false;
     ctx->work.pending = false;
+    dymu_internal_unmark_slots(ctx, 0, 1);
     return dymu_internal_fill(ctx, ctx->T, 1.0 / 0.0, (size_t)ctx->pitch * ctx->rows);
 }
 
@@ -1742,6 +1760,7 @@ int dymu_import_rows_min_key(dymu_ctx* ctx, uint32_t slot, uint32_t j0, uint32_t
         || (uint64_t)j0 + n_rows > ctx->ny)
         return DYMU_ERR_ARG;
     DYMU_TRY(dymu_internal_settle_delivery(ctx));
+    dymu_internal_unmark_slots(ctx, slot, 1);
     size_t bytes = (size_t)ctx->nx * n_rows * sizeof(double);
     DYMU_TRY(dymu_internal_scratch(ctx, bytes + 64, device_ptr ? 64 : bytes + 64));
     int* d_flag = (int*)ctx->d_scratch;

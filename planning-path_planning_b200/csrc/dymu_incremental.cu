@@ -193,6 +193,7 @@ int dymu_solve_incremental(dymu_ctx* ctx, uint32_t goal_i, uint32_t goal_j, dymu
                           && ctx->last_goal_j == goal_j && !ctx->work.unclean && ctx->have_cost
                           && n < ((size_t)1 << 32);
     if (!reusable) return dymu_solve_total_cost(ctx, 1, &goal_i, &goal_j, stats);
+    dymu_internal_unmark_slots(ctx, 0, 1);
     if (stats) memset(stats, 0, sizeof(*stats));
     // (an unchanged map keeps a matrix that was delivered directly; a partial re-solve does not)
     if (!ctx->ceff_dirty)

@@ -402,6 +402,20 @@ int dymu_batch_solve_maps(dymu_ctx** ctxs, uint32_t n_ctx, uint32_t n_maps, cons
         if (c->aniso_n || c->clear_on)
             DYMU_FAIL(c, DYMU_ERR_STATE, "context %u: map batches are isotropic and without obstacle clearance", k);
     }
+    // every context solves with its own batch settings: they have to be the same everywhere
+    const dymu_ctx* c0 = ctxs[0];
+    for (uint32_t k = 1; k < n_ctx; ++k)
+    {
+        const dymu_ctx* c = ctxs[k];
+        bool same = c->mclear_on == c0->mclear_on && c->maniso_n == c0->maniso_n;
+        if (same && c0->mclear_on)
+            same = c->mclear_radius == c0->mclear_radius && c->mclear_margin == c0->mclear_margin
+                   && c->mclear_penalty == c0->mclear_penalty;
+        for (int e = 0; e < c0->maniso_n && same; ++e)
+            same = c->maniso_theta[e] == c0->maniso_theta[e] && c->maniso_f[e] == c0->maniso_f[e];
+        if (!same)
+            DYMU_FAIL(ctxs[k], DYMU_ERR_ARG, "context %u: its batch clearance or anisotropy differs from context 0's", k);
+    }
     if (n_maps == 0) return DYMU_OK;
     BatchShared S;
     S.ctxs = ctxs; S.n_ctx = n_ctx; S.n_goals = n_maps; S.goal_i = goal_i; S.goal_j = goal_j;

@@ -19,7 +19,8 @@
 // of queries run one CTA per query.
 // With slope anisotropy on (dymu_set_anisotropy) the helpers put the characteristic direction
 // of the anisotropic metric into the window instead of the normalised gradient; the walker is
-// the same.
+// the same.  On a slot written by an anisotropic map solve (dymu_set_maps_anisotropy) the helpers
+// build each directional cost from the map's cost-term plane and the batch factor planes instead.
 #include <limits.h>
 #include <type_traits>
 #include <stdio.h>
@@ -60,6 +61,15 @@ struct PathArgsAniso : PathArgs
 {
     const double* A;
     size_t a_stride;  // doubles between two of those planes
+};
+
+// the descent on a slot of an anisotropic map solve: a(x->m) = C(x) * F_d(x), C the map's cost-term
+// plane (clearance-adjusted or plain, as the solve used it), F the four factor planes of the batch
+struct PathArgsMaps : PathArgs
+{
+    const double* C;
+    const double* F;
+    size_t f_stride;  // doubles between two factor planes
 };
 
 // per-axis rule of gradientNode (G.cpp:722-761); lo/hi missing = NULL neighbour
@@ -138,7 +148,16 @@ __device__ __forceinline__ void build_window(const Args& a, double* wb, int x0, 
                 if (hr[u]) fr[u] = __ldcg(Tc + 1);
                 if (hd[u]) fd[u] = __ldcg(Tc - a.pitch);
                 if (hu[u]) fu[u] = __ldcg(Tc + a.pitch);
-                if constexpr (ANISO)
+                if constexpr (std::is_same<Args, PathArgsMaps>::value)
+                {
+                    // the solver's C_q(x) * F_d(x), bit for bit
+                    const double c = __ldg(a.C + at);
+                    axm[u] = c * __ldg(a.F + at);
+                    axp[u] = c * __ldg(a.F + a.f_stride + at);
+                    aym[u] = c * __ldg(a.F + 2 * a.f_stride + at);
+                    ayp[u] = c * __ldg(a.F + 3 * a.f_stride + at);
+                }
+                else if constexpr (ANISO)
                 {
                     axm[u] = __ldg(a.A + at);
                     axp[u] = __ldg(a.A + a.a_stride + at);
@@ -445,26 +464,58 @@ __global__ void __launch_bounds__(PATH_THREADS, 1) k_global_path(const Args* arg
 
 template <class Args> int launch_paths_as(dymu_ctx* ctx, uint32_t n, const Args* d_args)
 {
-    constexpr bool aniso = std::is_same<Args, PathArgsAniso>::value;
-    auto kernel = (ctx->gres == 1.0) ? k_global_path<true, aniso> : k_global_path<false, aniso>;
+    constexpr bool aniso = !std::is_same<Args, PathArgs>::value;
+    auto kernel = (ctx->gres == 1.0) ? k_global_path<true, aniso, Args> : k_global_path<false, aniso, Args>;
     DYMU_CUDA_TRY(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PATH_SMEM));
     kernel<<<n, PATH_THREADS, PATH_SMEM, ctx->stream>>>(d_args);
     return DYMU_OK;
 }
 
-// d_args: n argument blocks of args_size(ctx) bytes each
-int launch_paths(dymu_ctx* ctx, uint32_t n, const void* d_args)
+// which descent a slot takes: the map-anisotropic one on a slot of an anisotropic map solve, otherwise
+// the context's (anisotropic while the context's anisotropy is on)
+enum Kind { kIso = 0, kAniso = 1, kMaps = 2 };
+Kind kind_of(const dymu_ctx* ctx, uint32_t slot)
 {
-    if (ctx->aniso_n) return launch_paths_as(ctx, n, (const PathArgsAniso*)d_args);
+    if (ctx->slot_mark && ctx->slot_mark[slot] == kSlotMapAniso) return kMaps;
+    return ctx->aniso_n ? kAniso : kIso;
+}
+
+// d_args: n argument blocks of args_size(kind) bytes each
+int launch_paths(dymu_ctx* ctx, Kind kind, uint32_t n, const void* d_args)
+{
+    if (kind == kMaps) return launch_paths_as(ctx, n, (const PathArgsMaps*)d_args);
+    if (kind == kAniso) return launch_paths_as(ctx, n, (const PathArgsAniso*)d_args);
     return launch_paths_as(ctx, n, (const PathArgs*)d_args);
 }
 
-size_t args_size(const dymu_ctx* ctx) { return ctx->aniso_n ? sizeof(PathArgsAniso) : sizeof(PathArgs); }
-
-// the argument block of one query in the form the kernel of the context's mode takes
-void put_args(const dymu_ctx* ctx, const PathArgs& a, void* dst)
+size_t args_size(Kind kind)
 {
-    if (ctx->aniso_n)
+    return kind == kMaps ? sizeof(PathArgsMaps) : kind == kAniso ? sizeof(PathArgsAniso) : sizeof(PathArgs);
+}
+
+// a slot whose anisotropic map solve no longer matches its planes has no descent
+int check_slot(dymu_ctx* ctx, uint32_t slot)
+{
+    if (ctx->slot_mark && ctx->slot_mark[slot] == kSlotMapAnisoStale)
+        DYMU_FAIL(ctx, DYMU_ERR_STATE, "slot %u: its anisotropic map solve is stale (the map was set again, the batch "
+                  "settings changed or the maps were reserved again)", slot);
+    return DYMU_OK;
+}
+
+// the argument block of one query on `slot` in the form the kernel of its kind takes
+void put_args(const dymu_ctx* ctx, Kind kind, uint32_t slot, const PathArgs& a, void* dst)
+{
+    if (kind == kMaps)
+    {
+        PathArgsMaps x;
+        static_cast<PathArgs&>(x) = a;
+        const size_t plane = (size_t)ctx->pitch * ctx->rows;
+        x.C = (ctx->mclear_on ? ctx->maps_adj : ctx->maps) + (size_t)slot * plane;
+        x.F = ctx->maps_fac;
+        x.f_stride = plane;
+        memcpy(dst, &x, sizeof(x));
+    }
+    else if (kind == kAniso)
     {
         PathArgsAniso x;
         static_cast<PathArgs&>(x) = a;
@@ -488,9 +539,11 @@ int dymu_extract_global_path(dymu_ctx* ctx, uint32_t slot, double x0, double y0,
     if (goal_i >= ctx->nx || goal_j >= ctx->ny) return DYMU_ERR_ARG;
     size_t out_bytes = (size_t)cap * 5 * sizeof(double);
     size_t hdr = 256;
-    if (ctx->aniso_n) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
+    DYMU_TRY(check_slot(ctx, slot));
+    const Kind kind = kind_of(ctx, slot);
+    if (kind == kAniso) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
     DYMU_TRY(dymu_internal_scratch(ctx, hdr + out_bytes, hdr + out_bytes));
-    const size_t asz = args_size(ctx);
+    const size_t asz = args_size(kind);
     PathArgs a;
     a.T = ctx->T + (size_t)slot * ctx->pitch * ctx->rows;
     a.elev = ctx->elev;
@@ -503,12 +556,14 @@ int dymu_extract_global_path(dymu_ctx* ctx, uint32_t slot, double x0, double y0,
 #ifdef DYMU_PATH_PROFILE
     a.prof = (unsigned long long*)((char*)ctx->d_scratch + asz + 8);
     static_assert(sizeof(PathArgsAniso) + 8 + 4 * 8 <= 256, "path header overflow");
+    static_assert(sizeof(PathArgsMaps) + 8 + 4 * 8 <= 256, "path header overflow");
 #else
     static_assert(sizeof(PathArgsAniso) + 8 <= 256, "path header overflow");
+    static_assert(sizeof(PathArgsMaps) + 8 <= 256, "path header overflow");
 #endif
-    put_args(ctx, a, ctx->h_pinned);
+    put_args(ctx, kind, slot, a, ctx->h_pinned);
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_scratch, ctx->h_pinned, asz, cudaMemcpyHostToDevice, ctx->stream));
-    DYMU_TRY(launch_paths(ctx, 1, ctx->d_scratch));
+    DYMU_TRY(launch_paths(ctx, kind, 1, ctx->d_scratch));
     ctx->launches++;
     DYMU_CUDA_TRY(ctx, cudaGetLastError());
     uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + asz);
@@ -545,16 +600,28 @@ int dymu_extract_global_path_batch(dymu_ctx* ctx, uint32_t n, const uint32_t* sl
     for (uint32_t q = 0; q < n; ++q)
         if (slots[q] >= ctx->n_slots || goal_ij[2 * q] >= ctx->nx || goal_ij[2 * q + 1] >= ctx->ny)
             return DYMU_ERR_ARG;
-    if (ctx->aniso_n) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
-    const size_t asz = args_size(ctx);
-    const size_t hdr = (((size_t)n * (asz + 8)) + 255) & ~(size_t)255;
+    for (uint32_t q = 0; q < n; ++q) DYMU_TRY(check_slot(ctx, slots[q]));
+    // queries on slots of anisotropic map solves take their own kernel: one launch per kind, each
+    // over its own run of argument blocks (the results stay in query order)
+    uint32_t n_kind[3] = {0, 0, 0};
+    for (uint32_t q = 0; q < n; ++q) n_kind[kind_of(ctx, slots[q])]++;
+    if (n_kind[kAniso]) DYMU_TRY(dymu_internal_refresh_ceff(ctx));  // the directional costs are current
+    size_t kind_off[3], args_bytes = 0;
+    for (int k = 0; k < 3; ++k)
+    {
+        kind_off[k] = args_bytes;
+        args_bytes += (size_t)n_kind[k] * args_size((Kind)k);
+    }
+    const size_t hdr = ((args_bytes + (size_t)n * 8) + 255) & ~(size_t)255;
     const size_t out_bytes = (size_t)n * cap * 5 * sizeof(double);
     DYMU_TRY(dymu_internal_scratch(ctx, hdr + out_bytes, hdr));
     char* h_args = (char*)ctx->h_pinned;
     char* d_base = (char*)ctx->d_scratch;
-    uint32_t* d_res = (uint32_t*)(d_base + (size_t)n * asz);
+    uint32_t* d_res = (uint32_t*)(d_base + args_bytes);
+    uint32_t at_kind[3] = {0, 0, 0};
     for (uint32_t q = 0; q < n; ++q)
     {
+        const Kind kind = kind_of(ctx, slots[q]);
         PathArgs a;
         a.T = ctx->T + (size_t)slots[q] * ctx->pitch * ctx->rows;
         a.elev = ctx->elev;
@@ -567,13 +634,17 @@ int dymu_extract_global_path_batch(dymu_ctx* ctx, uint32_t n, const uint32_t* sl
 #ifdef DYMU_PATH_PROFILE
         a.prof = nullptr;
 #endif
-        put_args(ctx, a, h_args + (size_t)q * asz);
+        put_args(ctx, kind, slots[q], a, h_args + kind_off[kind] + (size_t)(at_kind[kind]++) * args_size(kind));
     }
-    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(d_base, h_args, (size_t)n * asz, cudaMemcpyHostToDevice, ctx->stream));
-    DYMU_TRY(launch_paths(ctx, n, d_base));
-    ctx->launches++;
-    DYMU_CUDA_TRY(ctx, cudaGetLastError());
-    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + (size_t)n * asz);
+    DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(d_base, h_args, args_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    for (int k = 0; k < 3; ++k)
+    {
+        if (!n_kind[k]) continue;
+        DYMU_TRY(launch_paths(ctx, (Kind)k, n_kind[k], d_base + kind_off[k]));
+        ctx->launches++;
+        DYMU_CUDA_TRY(ctx, cudaGetLastError());
+    }
+    uint32_t* h_res = (uint32_t*)((char*)ctx->h_pinned + args_bytes);
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h_res, d_res, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (uint32_t q = 0; q < n; ++q)

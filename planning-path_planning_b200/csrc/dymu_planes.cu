@@ -328,6 +328,36 @@ __global__ void k_dircost(const double* __restrict__ elev, const double* __restr
     }
 }
 
+// Factor planes of the anisotropic map batch (dymu_set_maps_anisotropy): k_dircost's factor alone,
+//     F_d(x) = f(atan((elev[m] - elev[x]) / gres) * (180/pi))
+// for every cell of the grid toward its neighbour m = i-1, i+1, j-1, j+1, +inf toward a neighbour
+// outside the grid and on the padding (never 0: the solver multiplies, and inf * 0 is NaN).  The
+// solver's C_q(x) * F_d(x) is then k_dircost's a(x->m) of map q bit for bit.  8 B read + 32 B
+// written per cell.
+__global__ void k_dirfactor(const double* __restrict__ elev, double* __restrict__ F, size_t plane, double gres,
+                            uint32_t pitch, uint32_t rows, uint32_t nx, uint32_t ny, AnisoTable tab)
+{
+    constexpr double kDeg = 180.0 / 3.141592653589793;
+    const size_t total = (size_t)pitch * rows;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < total; q += stride)
+    {
+        const uint32_t j = (uint32_t)(q / pitch), i = (uint32_t)(q % pitch);
+        double a[4] = {DYMU_INF, DYMU_INF, DYMU_INF, DYMU_INF};
+        if (i < nx && j < ny)
+        {
+            const double e = elev[q];
+            const bool has[4] = {i > 0, i + 1 < nx, j > 0, j + 1 < ny};
+            const ptrdiff_t off[4] = {-1, 1, -(ptrdiff_t)pitch, (ptrdiff_t)pitch};
+#pragma unroll
+            for (int d = 0; d < 4; ++d)
+                if (has[d]) a[d] = aniso_factor(tab, atan((elev[q + off[d]] - e) / gres) * kDeg);
+        }
+#pragma unroll
+        for (int d = 0; d < 4; ++d) F[d * plane + q] = a[d];
+    }
+}
+
 // dense read-back with the getter transforms of G.cpp:799-829.  8(+17) B read, 8 B written.
 __global__ void k_readback(const double* __restrict__ src, const double* __restrict__ haz,
                            const double* __restrict__ traff, const uint8_t* __restrict__ obst,
@@ -584,6 +614,7 @@ int dymu_destroy(dymu_ctx* ctx)
     if (ctx->ev_tail) cudaEventDestroy(ctx->ev_tail);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
+    dymu_internal_unmark_all(ctx);
     free(ctx);
     return DYMU_OK;
 }
@@ -1171,6 +1202,24 @@ static int build_dircost(dymu_ctx* ctx)
     DYMU_CUDA_TRY(ctx, cudaMemcpyAsync(h, d, 16, cudaMemcpyDeviceToHost, ctx->stream));
     DYMU_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->aniso_band = h[1] > 0 ? kBandFactor * (double)kTile * (h[0] / h[1]) : 1.0 / 0.0;
+    return DYMU_OK;
+}
+
+int dymu_internal_maps_factors(dymu_ctx* ctx)
+{
+    const size_t n = (size_t)ctx->pitch * ctx->rows;
+    AnisoTable tab;
+    tab.n = ctx->maniso_n;
+    for (int k = 0; k < DYMU_ANISO_MAX; ++k)
+    {
+        tab.theta[k] = k < tab.n ? ctx->maniso_theta[k] : 0.0;
+        tab.f[k] = k < tab.n ? ctx->maniso_f[k] : 0.0;
+    }
+    if (!ctx->maps_fac) DYMU_CUDA_TRY(ctx, cudaMalloc((void**)&ctx->maps_fac, 4 * n * sizeof(double)));
+    k_dirfactor<<<stream_grid(ctx, n), kThreads, 0, ctx->stream>>>(ctx->elev, ctx->maps_fac, n, ctx->gres, ctx->pitch,
+                                                                   ctx->rows, ctx->nx, ctx->ny, tab);
+    ctx->launches++;
+    DYMU_CUDA_TRY(ctx, cudaGetLastError());
     return DYMU_OK;
 }
 

@@ -83,6 +83,8 @@ _SIG = {
     "dymu_batch_solve_maps": (C.c_int, [C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, _dp, C.c_size_t, C.c_size_t,
                                         _u32p, _u32p, _dp, C.c_double, _dp, C.c_uint32, _u32p,
                                         C.POINTER(C.c_int32), _dp, C.c_size_t, C.POINTER(C.c_float)]),
+    "dymu_set_maps_clearance": (C.c_int, [C.c_void_p, C.c_double, C.c_double, C.c_double]),
+    "dymu_set_maps_anisotropy": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int]),
     "dymu_local_reshape": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int64, C.c_int64]),
     "dymu_solve_incremental": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(SolveStats),
                                          C.POINTER(C.c_uint64)]),
@@ -345,6 +347,19 @@ class DeviceLayer:
         self._chk(self._l.dymu_solve_maps(self._h, g.shape[0], gi.ctypes.data_as(_u32p), gj.ctypes.data_as(_u32p),
                                           C.byref(st)))
         return st.as_dict()
+
+    def set_maps_clearance(self, radius, margin, penalty):
+        """Obstacle clearance of every map solve of this layer (the obstacles of map q are its cells with
+        cost <= 0); parameters as set_obstacle_clearance, (0, 0, 0) switches it off."""
+        self._chk(self._l.dymu_set_maps_clearance(self._h, float(radius), float(margin), float(penalty)))
+
+    def set_maps_anisotropy(self, theta_deg, factors):
+        """Slope anisotropy of every map solve of this layer, on the layer's elevation plane; table as
+        set_anisotropy, empty tables switch it off."""
+        t, f = _f64(theta_deg).ravel(), _f64(factors).ravel()
+        if t.size != f.size:
+            raise ValueError("theta_deg and factors differ in length")
+        self._chk(self._l.dymu_set_maps_anisotropy(self._h, t.ctypes.data_as(_dp), f.ctypes.data_as(_dp), t.size))
 
     def solve_incremental(self, goal):
         """Re-solve after small changes of cost / hazard_density / trafficability.  Returns
